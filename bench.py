@@ -13,6 +13,11 @@ checks 8 streams of every rank's shard against the CPU oracle outside the timed 
 roofline entry per kernel from separate profiling passes, and measures end to end through the C multi-GPU host
 (fmb_multi: one process, one worker thread per device, one pinned buffer) next to the box's raw copy ceiling.
 Prints ONE JSON line on rank 0.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs bench_outputs
+
+also writes the PCM of the headline's last timed step, as float32 .npy files (see dump_outputs), so that two
+builds run with the same arguments -- hence the same synthetic inputs -- can be compared output for output.
 """
 from __future__ import annotations
 
@@ -277,7 +282,7 @@ def run_ours(args):
         host_group = dist.new_group(backend="gloo")       # host-side barriers/gathers that must not touch the GPUs
     red_dev = "cuda" if dist is None or dist.get_backend() == "nccl" else "cpu"
 
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     stereo = args.mode == "stereo"
     mk = R.DemodConfig.stereo_192k if stereo else R.DemodConfig.mono_192k
     okw = dict(rate_in=192000, rate_out2=48000, mode=2 if stereo else 1, size=90 if stereo else 128)
@@ -320,7 +325,7 @@ def run_ours(args):
 
     def time_resident(S, precision):
         """K timed steps of S streams per GPU, inputs resident in HBM; returns (ms over the K steps as max over
-        ranks, host enqueue seconds, launches, clocks)."""
+        ranks, host enqueue seconds, launches, clocks, PCM count per stream of the last step)."""
         fb = R.FmBatch(mk(n_streams=S, device=local, precision=precision, segments=args.segments))
         n_out = fb.next_out_count()
         pitch = (n_out + 7) & ~7
@@ -337,6 +342,8 @@ def run_ours(args):
             e0.record()
             t_host = time.perf_counter()
             for i in range(K):
+                if i == K - 1:
+                    n_last = fb.next_out_count()           # PCM per stream of the last step (host arithmetic)
                 fb.process_device(dev_in[(W + i) % args.nbuf].data_ptr(), BLOCK, dev_pcm.data_ptr(), pitch, stream)
             t_host = time.perf_counter() - t_host       # host time to enqueue the K steps (must stay below the device time)
             fb.join(stream)
@@ -344,11 +351,12 @@ def run_ours(args):
             barrier()
         ms = max_over_ranks(e0.elapsed_time(e1))
         launches = R.launch_count() - launches0
-        return fb, dev_in, dev_pcm, pitch, n_out, ms, t_host, launches, clk.summary()
+        return fb, dev_in, dev_pcm, pitch, n_out, ms, t_host, launches, clk.summary(), n_last
 
     # ---- headline: device-resident `value` ----
-    fb, dev_in, dev_pcm, pitch, n_out, ms_total, t_host, launches, clocks = time_resident(S_head, prec)
+    fb, dev_in, dev_pcm, pitch, n_out, ms_total, t_host, launches, clocks, n_last = time_resident(S_head, prec)
     value = S_head * world * SAMPLES_PER_BLOCK * K / (ms_total * 1e-3) * 1e-6
+    last_pcm = dev_pcm[:, :n_last].cpu().numpy() if args.dump_outputs else None   # the passes below overwrite dev_pcm
 
     # ---- per-kernel device times, in SEPARATE passes over the same steps (nothing below touches the headline):
     #   pass A: K pipelined steps with an event pair around every demod launch (its steady-state duration)
@@ -425,7 +433,7 @@ def run_ours(args):
             other = {"streams_per_gpu": S_other, "value": value, "ms_per_step": ms_total / K, "parity": parity_ok,
                      "note": "same shard size as the headline at this GPU count: one measurement"}
         else:
-            fb_o, _, _, _, _, ms_o, _, _, _ = time_resident(S_other, prec)
+            fb_o, _, _, _, _, ms_o, _, _, _, _ = time_resident(S_other, prec)
             fb_o.close()
             ok_o, _ = shard_parity(S_other)
             other = {"streams_per_gpu": S_other, "value": S_other * world * SAMPLES_PER_BLOCK * K / (ms_o * 1e-3) * 1e-6,
@@ -437,7 +445,7 @@ def run_ours(args):
     # tolerance north_star states for the floating-point stages); reported beside the bit-exact headline ----
     fma_alt = None
     if args.precision == "exact" and not args.no_fma_alt:
-        fb2, _, _, _, _, fma_ms, _, _, _ = time_resident(S_head, R.FMB_PRECISION_FMA)
+        fb2, _, _, _, _, fma_ms, _, _, _, _ = time_resident(S_head, R.FMB_PRECISION_FMA)
         fb2.close()
         fma_alt = {"value": S_head * world * SAMPLES_PER_BLOCK * K / (fma_ms * 1e-3) * 1e-6, "unit": UNIT, "ms_per_step": fma_ms / K,
                    "tolerance": "+-1 LSB int16 PCM vs the reference (tests/test_gpu_parity.py::test_fma_precision_within_one_lsb)"}
@@ -565,6 +573,8 @@ def run_ours(args):
             e2e["copy_ceiling"] = {"error": str(ex_)}
             e2e["copy_ceiling_frac"] = None
 
+    if last_pcm is not None:                              # every rank writes its own shard
+        dump_outputs(args.dump_outputs, last_pcm, "pcm" if world == 1 else f"pcm_rank{rank}", DUMP_BYTES // world)
     if rank != 0:
         if dist is not None:
             dist.barrier(group=host_group)
@@ -631,6 +641,21 @@ def run_ours(args):
     return 0
 
 
+DUMP_BYTES = 64_000_000           # --dump-outputs: at most this much in all
+
+
+def dump_outputs(out_dir: str, pcm: np.ndarray, name: str, budget: int) -> None:
+    """PCM [streams, samples] of one step -> out_dir/<name>.npy (float32, exact for int16) and
+    out_dir/<name>_streams.npy (float64 stream indices of its rows).  A batch that would take more than `budget`
+    bytes is cut to a fixed, seeded sample of whole streams."""
+    S, n = pcm.shape
+    keep = max(1, (budget - 256) // (n * 4 + 8))          # a float32 row + its float64 index; 256 B for two headers
+    rows = np.arange(S) if keep >= S else np.sort(np.random.default_rng(0).choice(S, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), pcm[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, f"{name}_streams.npy"), rows.astype(np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -668,7 +693,13 @@ def main():
     ap.add_argument("--no-fma-alt", action="store_true", help="skip the extra FMB_PRECISION_FMA timing")
     ap.add_argument("--no-other-scaling", action="store_true", help="skip the second (strong resp. weak) measurement")
     ap.add_argument("--no-e2e-per-process", action="store_true", help="skip the per-process end-to-end layout at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the PCM of the headline's last timed step to DIR/*.npy (float32, at most 64 MiB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

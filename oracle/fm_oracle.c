@@ -150,6 +150,16 @@ void fmo_get_state(void *h, struct fmo_state *out, int *phase, uint64_t *blocks)
     if (blocks) *blocks = o->blocks_done;
 }
 
+/* Restores a state fmo_get_state returned: the CPU side of hand-over tests, e.g. a stream that
+ * carries on under another volume. */
+void fmo_set_state(void *h, const struct fmo_state *in, int phase, uint64_t blocks)
+{
+    struct fmo *o = h;
+    o->st = *in;
+    o->resamp_phase = phase;
+    o->blocks_done = blocks;
+}
+
 /* ---- stage helpers ---- */
 
 /* Discriminator angle, :606-667.  Eight octant formulas, kept as separate

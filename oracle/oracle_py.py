@@ -69,6 +69,7 @@ class PortOracle:
         self.lib.fmo_bench.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_int]
         self.lib.fmo_get_tables.argtypes = [C.c_void_p] + [C.c_void_p] * 5
         self.lib.fmo_get_state.argtypes = [C.c_void_p, C.POINTER(PortState), C.POINTER(C.c_int), C.POINTER(C.c_uint64)]
+        self.lib.fmo_set_state.argtypes = [C.c_void_p, C.POINTER(PortState), C.c_int, C.c_uint64]
         self.cfg = _PortCfg(rate_in, rate_out2, mode, size, offset_tuning, deemph, volume, inplace_quirk, rate_out)
         self.h = self.lib.fmo_create(C.byref(self.cfg))
         if not self.h:
@@ -115,6 +116,9 @@ class PortOracle:
         st, ph, bl = PortState(), C.c_int(0), C.c_uint64(0)
         self.lib.fmo_get_state(self.h, C.byref(st), C.byref(ph), C.byref(bl))
         return st, ph.value, bl.value
+
+    def set_state(self, st: PortState, phase: int, blocks: int) -> None:
+        self.lib.fmo_set_state(self.h, C.byref(st), phase, blocks)
 
 
 def ref_available() -> bool:

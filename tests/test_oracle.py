@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 from oracle.oracle_py import PortOracle, RefOracle, ref_available
-from vectors import B, CASES, CONFIGS, LONG_CASES, long_capture_bytes, make_input, sha
+from vectors import B, CASE_BY_ID, CASES, CONFIGS, LONG_CASES, long_capture_bytes, make_input, sha
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = np.load(os.path.join(HERE, "golden", "golden.npz"))
@@ -89,15 +89,19 @@ def test_known_constants_from_survey():
     assert m[3] == np.float32(0.4) * np.float32(32768.0)
 
 
-@pytest.mark.skipif(not ref_available(), reason="oracle/_ref not built")
 def test_rate_out_differs_from_rate_in_under_post_downsample():
     """-o N: main does rate_in *= post_downsample (:1510) and leaves rate_out, so the filters are designed for
-    rate_in while lp_real_f32's ticks run at rate_out/rate_out2 (:485).  The port follows the reference there,
-    and the result is NOT what rate_out = rate_in would give."""
+    rate_in while lp_real_f32's ticks run at rate_out/rate_out2 (:485).  The port follows the reference there
+    (the reference's PCM of the golden case stereo384_o2_fm, and the live reference where it is built), and the
+    result is NOT what rate_out = rate_in would give."""
     kw = CONFIGS["stereo384_o2"]
-    iq = make_input("stereo384_o2", "fm_stereo", 1, 2)
-    a = RefOracle(**kw).run(iq)
+    cid, cfg, kind, stream, blocks = CASE_BY_ID["stereo384_o2_fm"]
+    iq = make_input(cfg, kind, stream, blocks)
+    a = GOLD[cid]
     assert np.array_equal(a, PortOracle(**kw).run(iq))
+    if ref_available():
+        live = make_input("stereo384_o2", "fm_stereo", 1, 2)
+        assert np.array_equal(RefOracle(**kw).run(live), PortOracle(**kw).run(live))
     same_rate = dict(kw, rate_out=0)
     assert PortOracle(**same_rate).run(iq).size != a.size     # 8 ticks per 64 samples instead of 16
 
