@@ -25,6 +25,21 @@
 #include <stdlib.h>
 #include <string.h>
 
+/*
+ * The FIR multiply-accumulate: the channel FIR's taps 1-15, the three decoder FIRs (vm, vp, vs) and
+ * the symmetric FIRs of the second low-pass and of mono.  Built plainly it is the reference's
+ * acc + x*c, product and sum rounded separately.  Built with -DFMO_FMA it is fmaf(x, c, acc), one
+ * rounding: the fused restatement, which defines FMB_PRECISION_FMA bit for bit.  Nothing else is
+ * fused in either build: the channel FIR's first tap stays a rounded product, and the pilot, the
+ * discriminator and de-emphasis keep every rounding.  fmaf is correctly rounded with or without
+ * hardware FMA, so the fused build needs no -mfma.
+ */
+#ifdef FMO_FMA
+#define FMO_MAC(x, c, acc) fmaf((x), (c), (acc))
+#else
+#define FMO_MAC(x, c, acc) ((acc) + (x) * (c))
+#endif
+
 #define FMO_HIST 128      /* >= largest supported FIR length - 1 */
 #define FMO_MAX_TAPS 64   /* size/2 */
 
@@ -200,7 +215,7 @@ static float sym_fir(const float *a, int n, int size, int taps, const float *c)
 {
     float acc = 0;
     int k;
-    for (k = 0; k < taps; k++) acc += (a[n - (size - 1) + k] + a[n - k]) * c[k];
+    for (k = 0; k < taps; k++) acc = FMO_MAC(a[n - (size - 1) + k] + a[n - k], c[k], acc);
     return acc;
 }
 
@@ -265,8 +280,8 @@ int fmo_block(void *h, const uint8_t *iq, uint32_t len, int16_t *pcm, float *dem
         float aq = (pq_[0] + pq_[31]) * o->chan[0];
         float y, x;
         for (t = 1; t < 16; t++) {
-            ai = ai + (pi_[t] + pi_[31 - t]) * o->chan[t];
-            aq = aq + (pq_[t] + pq_[31 - t]) * o->chan[t];
+            ai = FMO_MAC(pi_[t] + pi_[31 - t], o->chan[t], ai);
+            aq = FMO_MAC(pq_[t] + pq_[31 - t], o->chan[t], aq);
         }
         y = st->pre_r * aq - st->pre_j * ai; /* :679 */
         x = ai * st->pre_r + aq * st->pre_j; /* :680 */
@@ -293,9 +308,9 @@ int fmo_block(void *h, const uint8_t *iq, uint32_t len, int16_t *pcm, float *dem
                 int k;
                 for (k = 0; k < T; k++) {
                     float v = hb[n - (S - 1) + k] + hb[n - k];
-                    vm += v * o->fm[k];
-                    vp += v * o->fp[k];
-                    vs += v * o->fs[k];
+                    vm = FMO_MAC(v, o->fm[k], vm);
+                    vp = FMO_MAC(v, o->fp[k], vp);
+                    vs = FMO_MAC(v, o->fs[k], vs);
                 }
                 hm[n] = vm;
                 hs[n] = vs * pilot_double(vp * o->swf, vp * o->cwf - st->pp);

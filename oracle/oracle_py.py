@@ -1,6 +1,8 @@
 """ctypes access to the two CPU checkers.  TEST INFRASTRUCTURE ONLY.
 
-  * `PortOracle`  -- oracle/libfm_oracle.so, our C restatement (oracle/fm_oracle.c)
+  * `PortOracle`  -- oracle/libfm_oracle.so, our C restatement (oracle/fm_oracle.c); with fma=True
+                     oracle/libfm_oracle_fma.so, the same built with FMO_FMA (FIR multiply-adds fused:
+                     the definition of FMB_PRECISION_FMA)
   * `RefOracle`   -- oracle/_ref/libfmref.so, the reference's own rtl_fm_player.c compiled
                      unmodified (oracle/ref_harness.c); built only where /root/reference exists,
                      the prebuilt file travels to the GPU box.
@@ -18,6 +20,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 PORT_PATH = os.path.join(_HERE, "libfm_oracle.so")
+PORT_FMA_PATH = os.path.join(_HERE, "libfm_oracle_fma.so")
 REF_PATH = os.path.join(_HERE, "_ref", "libfmref.so")
 REF_CLI = os.path.join(_HERE, "_ref", "ref_offline")
 REF_BLOCK = 262144
@@ -51,13 +54,14 @@ def _f32(n):
 
 
 class PortOracle:
-    """One channel of the C restatement."""
+    """One channel of the C restatement; fma=True: its fused build, the model of FMB_PRECISION_FMA."""
 
     def __init__(self, rate_in=240000, rate_out2=48000, mode=2, size=90, offset_tuning=0, deemph=0.000050,
-                 volume=0.4, inplace_quirk=1, rate_out=0):
-        if not os.path.exists(PORT_PATH):
+                 volume=0.4, inplace_quirk=1, rate_out=0, fma=False):
+        path = PORT_FMA_PATH if fma else PORT_PATH
+        if not os.path.exists(path):
             build("port")
-        self.lib = C.CDLL(PORT_PATH)
+        self.lib = C.CDLL(path)
         self.lib.fmo_create.restype = C.c_void_p
         self.lib.fmo_create.argtypes = [C.POINTER(_PortCfg)]
         self.lib.fmo_destroy.argtypes = [C.c_void_p]

@@ -166,22 +166,23 @@ def sweep_phases(kw, limit=500, sample=100, edges=40, seed=1):
     return out
 
 
-def run_phase_sweep(kw, phases, n, uniq, kind, ws_generic=True, bb=B):
+def run_phase_sweep(kw, phases, n, uniq, kind, ws_generic=True, bb=B, fma=False):
     """At every phase: the oracle and the handle are put into the same carried state and phase (fmo_set_state,
     fmb_set_state) and run one or two blocks; PCM, out counts, the next phase and, for few streams, the discriminator
     and decoder outputs must match.  The handle resumes twice from the same point: from a state built from the
     oracle's floats (raw_valid 0: chan_fir_from_state) and from the state it exported itself (raw_valid 1: raw tail).
-    Returns (ran, refused)."""
+    fma: the handle runs FMB_PRECISION_FMA and the oracle is the fused restatement.  Returns (ran, refused)."""
     mode, fast = kw["mode"], fast_of(kw)
     per = 2 if len(phases) <= 64 else 1
     nb = 3
     iq_u = np.stack([capture(kw, kind, s, (nb + per) * bb) for s in range(uniq)])
     rows = np.arange(n) % uniq
     blocks = [np.ascontiguousarray(iq_u[rows, b * bb:(b + 1) * bb]) for b in range(nb + per)]
-    orc = [PortOracle(**kw) for _ in range(uniq)]
+    orc = [PortOracle(**kw, fma=fma) for _ in range(uniq)]
     debug = n <= 4
     ran = refused_n = 0
-    with R.FmBatch(make_cfg(kw, n_streams=n, block_bytes=bb)) as fb:
+    precision = R.FMB_PRECISION_FMA if fma else R.FMB_PRECISION_EXACT
+    with R.FmBatch(make_cfg(kw, n_streams=n, block_bytes=bb, precision=precision)) as fb:
         if debug:
             fb.debug_enable(True)
         pcm = fb.process(blocks[0])                              # non-trivial history in every stage
@@ -365,36 +366,42 @@ BLOCK_K = [1, 2, 3, 5, 7, 8, 9, 16]
 BLOCK_CFGS = ["stereo192", "stereo192_128", "stereo240", "stereo170_44", "mono192", "mono240_32"]
 
 
-@pytest.mark.parametrize("k", BLOCK_K)
-@pytest.mark.parametrize("name", BLOCK_CFGS)
-def test_block_size_sweep(monkeypatch, name, k):
+def run_block_size_sweep(monkeypatch, kw, k, fma=False):
     """block_bytes = 32768*k: k sub-tiles per stream and block.  Several carried blocks against
     PortOracle.run(block_bytes=...), for every `segments` that divides k (and the automatic choice) on a few streams,
-    and for a batch with more units than resident CTAs handed out through the ticket counter in 1-sub-tile runs."""
-    kw = OFFGRID[name]
+    and for a batch with more units than resident CTAs handed out through the ticket counter in 1-sub-tile runs.
+    fma: FMB_PRECISION_FMA against the fused restatement.  Returns (segments values, batch streams)."""
     bb = QUANTUM * k
     nblk = 6
     kind = "fm_stereo" if kw["mode"] == 2 else "fm_mono"
+    precision = R.FMB_PRECISION_FMA if fma else R.FMB_PRECISION_EXACT
     iq = np.stack([capture(kw, kind if s % 2 == 0 else "random", s, nblk * bb) for s in range(4)])
-    want = [PortOracle(**kw).run(iq[s], block_bytes=bb) for s in range(4)]
+    want = [PortOracle(**kw, fma=fma).run(iq[s], block_bytes=bb) for s in range(4)]
     ref_pin(kw, iq[0], bb)
-    segs = [0] + [s for s in (1, 2, 4, 8, k) if k % s == 0]
-    for seg in sorted(set(segs)):
-        with R.FmBatch(make_cfg(kw, n_streams=3, block_bytes=bb, segments=seg)) as fb:
+    segs = sorted(set([0] + [s for s in (1, 2, 4, 8, k) if k % s == 0]))
+    for seg in segs:
+        with R.FmBatch(make_cfg(kw, n_streams=3, block_bytes=bb, segments=seg, precision=precision)) as fb:
             if kw["mode"] == 1:             # a forced segmentation has no warp-specialised plan
                 assert fb.kernel_name() == ("fmb_mono_ws_kernel" if seg == 0 else "fmb_demod_kernel")
             pcm = fb.run(iq[:3])
         for s in range(3):
-            assert np.array_equal(pcm[s], want[s]), (name, k, seg, s)
+            assert np.array_equal(pcm[s], want[s]), (k, seg, s)
     monkeypatch.setenv("FMB_CHUNK", "1")
     monkeypatch.setenv("FMB_TAIL_PCT", "50")
     n = -(-1024 // k)
     rows = np.arange(n) % 4
-    with R.FmBatch(make_cfg(kw, n_streams=n, block_bytes=bb)) as fb:
+    with R.FmBatch(make_cfg(kw, n_streams=n, block_bytes=bb, precision=precision)) as fb:
         got = [fb.process(np.ascontiguousarray(iq[rows, b * bb:(b + 1) * bb])) for b in range(4)]
     got = np.concatenate(got, axis=1)
     for s in range(n):
-        assert np.array_equal(got[s], want[s % 4][:got.shape[1]]), (name, k, "batch", s)
+        assert np.array_equal(got[s], want[s % 4][:got.shape[1]]), (k, "batch", s)
+    return segs, n
+
+
+@pytest.mark.parametrize("k", BLOCK_K)
+@pytest.mark.parametrize("name", BLOCK_CFGS)
+def test_block_size_sweep(monkeypatch, name, k):
+    run_block_size_sweep(monkeypatch, OFFGRID[name], k)
 
 
 # ---- 4. rate boundaries -------------------------------------------------------------------------------------------

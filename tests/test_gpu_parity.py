@@ -417,17 +417,23 @@ def test_back_to_back_launches_of_a_full_batch_overlap_and_stay_exact(monkeypatc
     is handed out whole through the ticket counter, the carried state and the decoder-output buffers are ordered per
     stream inside the kernels.  mono192 runs the warp-specialised kernel, stereo240 the in-place quirk, mono240 the
     generic tick path.  16 distinct channels against the oracle, every replica identical to its original."""
+    run_back_to_back(monkeypatch, cfgname, kind, pdl)
+
+
+def run_back_to_back(monkeypatch, cfgname, kind, pdl, fma=False):
+    """fma: FMB_PRECISION_FMA against the fused restatement."""
     import torch
     monkeypatch.setenv("FMB_PDL", pdl)
     n, uniq, blocks = 1024, 16, 6
     c = CONFIGS[cfgname]
+    precision = R.FMB_PRECISION_FMA if fma else R.FMB_PRECISION_EXACT
     iq_u = np.stack([make_input(cfgname, kind, s, blocks) for s in range(uniq)])
     d_u = torch.from_numpy(iq_u).cuda()
     idx = torch.arange(n, device="cuda") % uniq
     d_in = [d_u[:, b * B:(b + 1) * B].index_select(0, idx).contiguous() for b in range(blocks)]
     st = torch.cuda.Stream()
     torch.cuda.synchronize()
-    with R.FmBatch(cfg_for(cfgname, n_streams=n)) as fb:
+    with R.FmBatch(cfg_for(cfgname, n_streams=n, precision=precision)) as fb:
         pitch = (fb.max_out + 7) & ~7
         d_out = torch.zeros((blocks, n, pitch), dtype=torch.int16, device="cuda")
         counts = []
@@ -440,7 +446,7 @@ def test_back_to_back_launches_of_a_full_batch_overlap_and_stay_exact(monkeypatc
         fb.get_state(0, 1)                               # reports a device-side hand-over time-out, if any
     got = np.concatenate([d_out[b, :, :counts[b]].cpu().numpy() for b in range(blocks)], axis=1)
     for s in range(uniq):
-        assert np.array_equal(got[s], PortOracle(**c).run(iq_u[s])), s
+        assert np.array_equal(got[s], PortOracle(**c, fma=fma).run(iq_u[s])), s
     assert np.array_equal(got.reshape(n // uniq, uniq, -1), np.broadcast_to(got[:uniq], (n // uniq, uniq, got.shape[1])))
 
 
