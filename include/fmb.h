@@ -2,9 +2,10 @@
  * fmb.h -- C ABI of the B200 batched FM demodulator ("fmb": FM batch).
  *
  * One handle demodulates n_streams independent FM channels.  Every call of
- * fmb_process*() consumes one block of rtl_sdr-format uint8 IQ per stream and
- * produces that block's 16-bit PCM per stream -- exactly what one iteration of
- * the reference's demod thread does for its single channel:
+ * fmb_process*() consumes one block of rtl_sdr-format uint8 IQ per stream (or n
+ * consecutive blocks, fmb_set_blocks_per_call) and produces that block's 16-bit
+ * PCM per stream -- exactly what one iteration of the reference's demod thread
+ * does for its single channel:
  *
  *     rotate_90_u8_f32(d) | u8_f32(d) ; full_demod(d)
  *                                   (reference src/rtl_fm_player.c:879-889)
@@ -74,6 +75,10 @@ typedef struct fmb_config {
     int rate_out;      /* demod.rate_out: the "fast" rate of lp_real_f32's resampler (:485).  0 (default) =
                           rate_in, as for every CLI setting but -o N (main: rate_in *= post_downsample, :1510,
                           so the filters are designed for rate_in while the ticks run at rate_out/rate_out2) */
+    int max_blocks_per_call; /* most consecutive blocks of block_bytes per stream one process/submit call may take
+                          (fmb_set_blocks_per_call); 0 (default) = 1.  Buffers are sized for it, and
+                          max_blocks_per_call * block_bytes must stay below 2^31.  A call of n blocks produces
+                          bit for bit what n calls of one block produce: block_bytes keeps its meaning            */
 } fmb_config;
 
 typedef struct fmb_handle fmb_handle;
@@ -102,15 +107,27 @@ int fmb_set_volume(fmb_handle *h, float volume);
  * as after demod_init + init_lp_real_f32 (:1156, :413). */
 int fmb_reset(fmb_handle *h);
 
+/* Blocks per stream each following process / submit call consumes, 1 <= n <= max_blocks_per_call (default: the
+ * maximum).  Takes effect from the next call, like fmb_set_volume; fmb_reset keeps it.  With n > 1 stream s's
+ * row is n * block_bytes contiguous bytes (iq_pitch >= n * block_bytes), its PCM is the concatenation of the n
+ * blocks' PCM, fmb_get_state afterwards equals the state after n one-block calls (blocks_done advances by n) and
+ * the debug taps cover the whole row. */
+int fmb_set_blocks_per_call(fmb_handle *h, int n);
+
 /* int16 values per stream the NEXT process call will produce (result_len of
- * full_demod, :603/:787).  Stereo counts L and R separately.  Same for all streams. */
+ * full_demod, :603/:787, summed over the call's blocks).  Stereo counts L and R separately.  Same for all
+ * streams. */
 int fmb_next_out_count(const fmb_handle *h);
-/* Upper bound of the above over all calls (use to size PCM buffers). */
+/* int16 values per stream the first n_blocks blocks of the next call produce (0 <= n_blocks <=
+ * max_blocks_per_call): the PCM of a stream whose capture ends after n_blocks blocks of that call is this prefix.
+ * fmb_next_out_count(h) == fmb_out_count_blocks(h, blocks per call). */
+int fmb_out_count_blocks(const fmb_handle *h, int n_blocks);
+/* Upper bound of fmb_next_out_count over all calls at max_blocks_per_call blocks (use to size PCM buffers). */
 int fmb_max_out_count(const fmb_handle *h);
 
 /*
  * Synchronous host call (the drop-in granularity): iq_host[s*iq_pitch ...] holds
- * block_bytes of IQ for stream s, pcm_host[s*pcm_pitch ...] receives int16 PCM
+ * block_bytes (times the blocks per call) of IQ for stream s, pcm_host[s*pcm_pitch ...] receives int16 PCM
  * (pcm_pitch in int16 units, >= fmb_next_out_count()).  n_out (may be NULL)
  * receives the count for each stream.  Copies H2D, runs the kernels, copies D2H,
  * waits.  Host memory may be pageable or pinned.
@@ -156,7 +173,8 @@ int fmb_sync(fmb_handle *h);
 /*
  * Pipelined host path (end-to-end number): submit enqueues H2D copy, kernels
  * and D2H copy of one block-step on internal streams and returns a ticket;
- * up to FMB_PIPE_DEPTH submits may be in flight.  Host buffers must stay valid
+ * up to FMB_PIPE_DEPTH submits may be in flight, each with the blocks per call that were set when it was
+ * submitted (fmb_wait reports that submit's count).  Host buffers must stay valid
  * until fmb_wait(ticket) returns and should be pinned (fmb_host_alloc) for the
  * copies to overlap.
  */
@@ -216,8 +234,8 @@ int fmb_set_state(fmb_handle *h, int first, int count, const fmb_stream_state *i
 int fmb_get_tables(const fmb_handle *h, float *fb, float *fm, float *fp, float *fs, float *misc);
 
 /* Debug taps of the last process call (device-resident copies kept only when
- * enabled): dem = discriminator output f32[n_streams][block_bytes/16],
- * lr = decoder output before de-emphasis f32[n_streams][n_out]. */
+ * enabled): dem = discriminator output f32[n_streams][n_blocks*block_bytes/16],
+ * lr = decoder output before de-emphasis f32[n_streams][n_out], n_blocks and n_out those of that call. */
 int fmb_debug_enable(fmb_handle *h, int on);
 int fmb_debug_read(fmb_handle *h, float *dem_host, size_t dem_pitch, float *lr_host, size_t lr_pitch);
 
@@ -229,7 +247,8 @@ int fmb_profile_read(fmb_handle *h, double ms_total[2], int launches[2]);
 
 /* Diagnostic: the de-emphasis kernel runs its recurrence speculatively in time and verifies it
  * (DESIGN.md "Kernel 2"); this is the number of 1024-value chunks, since fmb_create, whose
- * verification failed and which were therefore redone sequentially.  Results are exact either way. */
+ * verification failed and which were therefore redone sequentially (on multi-block rows also the chunks of
+ * every time segment whose assumed start state was not its predecessor's end).  Results are exact either way. */
 int fmb_deemph_fallbacks(fmb_handle *h, unsigned long long *count);
 
 const char *fmb_last_error(void);

@@ -46,6 +46,9 @@ fmb_handle *fmb_multi_handle(fmb_multi *m, int shard);
 
 int fmb_multi_next_out_count(const fmb_multi *m);
 int fmb_multi_max_out_count(const fmb_multi *m);
+/* fmb_set_blocks_per_call / fmb_out_count_blocks for every shard: iq_host rows then hold n * block_bytes */
+int fmb_multi_set_blocks_per_call(fmb_multi *m, int n);
+int fmb_multi_out_count_blocks(const fmb_multi *m, int n_blocks);
 int fmb_multi_reset(fmb_multi *m);
 
 /* As fmb_submit / fmb_wait / fmb_process, for the whole batch: iq_host[s*iq_pitch ...] is stream s's

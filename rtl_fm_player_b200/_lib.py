@@ -28,7 +28,7 @@ class FmbConfig(C.Structure):
         ("offset_tuning", C.c_int), ("deemph", C.c_double), ("volume", C.c_float),
         ("n_streams", C.c_int), ("block_bytes", C.c_int), ("device", C.c_int),
         ("precision", C.c_int), ("segments", C.c_int), ("emulate_inplace_quirk", C.c_int),
-        ("deemph_lambda", C.c_float), ("rate_out", C.c_int),
+        ("deemph_lambda", C.c_float), ("rate_out", C.c_int), ("max_blocks_per_call", C.c_int),
     ]
 
 
@@ -60,6 +60,8 @@ SIGNATURES = {
     "fmb_reset": (C.c_int, [C.c_void_p]),
     "fmb_set_volume": (C.c_int, [C.c_void_p, C.c_float]),
     "fmb_next_out_count": (C.c_int, [C.c_void_p]),
+    "fmb_set_blocks_per_call": (C.c_int, [C.c_void_p, C.c_int]),
+    "fmb_out_count_blocks": (C.c_int, [C.c_void_p, C.c_int]),
     "fmb_max_out_count": (C.c_int, [C.c_void_p]),
     "fmb_process": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),
     "fmb_process_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
@@ -94,6 +96,8 @@ SIGNATURES = {
     "fmb_multi_shard_range": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "fmb_multi_handle": (C.c_void_p, [C.c_void_p, C.c_int]),
     "fmb_multi_next_out_count": (C.c_int, [C.c_void_p]),
+    "fmb_multi_set_blocks_per_call": (C.c_int, [C.c_void_p, C.c_int]),
+    "fmb_multi_out_count_blocks": (C.c_int, [C.c_void_p, C.c_int]),
     "fmb_multi_max_out_count": (C.c_int, [C.c_void_p]),
     "fmb_multi_reset": (C.c_int, [C.c_void_p]),
     "fmb_multi_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),

@@ -35,6 +35,7 @@ class DemodConfig:
     emulate_inplace_quirk: int = 1
     deemph_lambda: float = 0.0
     rate_out: int = 0          # demod.rate_out (the resampler's fast rate, :485); 0 = rate_in
+    max_blocks_per_call: int = 0   # most consecutive blocks per stream one call may take; 0 = 1
 
     @classmethod
     def stereo_192k(cls, **kw) -> "DemodConfig":
@@ -60,6 +61,10 @@ class DemodConfig:
     def iq_samples_per_block(self) -> int:
         return self.block_bytes // 2
 
+    @property
+    def max_blocks(self) -> int:
+        return max(1, self.max_blocks_per_call)
+
 
 class FmBatch:
     """n_streams demodulators behind one handle (fmb_create / fmb_process / fmb_destroy)."""
@@ -71,6 +76,8 @@ class FmBatch:
         cc = cfg.to_c()
         L.check(self._lib.fmb_create(C.byref(cc), C.byref(self._h)), "fmb_create")
         self.max_out = self._lib.fmb_max_out_count(self._h)
+        self._blocks = cfg.max_blocks          # blocks per call, as fmb_create leaves it
+        self._last_blocks = 1
 
     # -- lifetime ---------------------------------------------------------------------------
     def close(self) -> None:
@@ -94,6 +101,15 @@ class FmBatch:
     def next_out_count(self) -> int:
         return L.check(self._lib.fmb_next_out_count(self._h), "fmb_next_out_count")
 
+    def set_blocks_per_call(self, n: int) -> None:
+        """Blocks per stream the following calls consume (1 .. max_blocks_per_call; default the maximum)."""
+        L.check(self._lib.fmb_set_blocks_per_call(self._h, n), "fmb_set_blocks_per_call")
+        self._blocks = n
+
+    def out_count_blocks(self, n_blocks: int) -> int:
+        """int16 values per stream the first n_blocks blocks of the next call produce."""
+        return L.check(self._lib.fmb_out_count_blocks(self._h, n_blocks), "fmb_out_count_blocks")
+
     def kernel_name(self) -> str:
         return self._lib.fmb_demod_kernel_name(self._h).decode()
 
@@ -114,22 +130,30 @@ class FmBatch:
 
     # -- host path (the drop-in granularity: one block per stream in, PCM out) --------------
     def process(self, iq: np.ndarray) -> np.ndarray:
-        """iq: uint8 [n_streams, block_bytes] -> int16 [n_streams, n_out] (fmb_process)."""
+        """iq: uint8 [n_streams, m * block_bytes], 1 <= m <= max_blocks_per_call, m consecutive blocks of each
+        stream -> int16 [n_streams, n_out] (fmb_process), the concatenation of the m blocks' PCM."""
+        m = iq.shape[1] // self.cfg.block_bytes if iq.ndim == 2 else 0
+        if m != self._blocks and 1 <= m <= self.cfg.max_blocks:
+            self.set_blocks_per_call(m)
         iq = self._check_iq(iq)
         n = self.next_out_count()
         pitch = max(8, (n + 7) & ~7)
         pcm = np.empty((self.cfg.n_streams, pitch), dtype=np.int16)
-        iq_pitch = iq.strides[0] if iq.shape[0] > 1 else self.cfg.block_bytes   # a 1-row view may carry stride 0
+        row = m * self.cfg.block_bytes
+        iq_pitch = iq.strides[0] if iq.shape[0] > 1 else row   # a 1-row view may carry stride 0
         L.check(self._lib.fmb_process(self._h, iq.ctypes.data, iq_pitch, pcm.ctypes.data, pitch, None),
                 "fmb_process")
+        self._last_blocks = m
         return pcm[:, :n]
 
     def run(self, iq: np.ndarray) -> np.ndarray:
         """Whole captures: uint8 [n_streams, n_bytes]; full blocks only, the short tail is
-        dropped as demod_thread_fn does (:863-868).  Returns int16 [n_streams, total]."""
+        dropped as demod_thread_fn does (:863-868).  Calls of max_blocks_per_call blocks, and a shorter
+        last one.  Returns int16 [n_streams, total]."""
         assert iq.ndim == 2 and iq.shape[0] == self.cfg.n_streams
-        bb = self.cfg.block_bytes
-        outs = [self.process(iq[:, b * bb:(b + 1) * bb]) for b in range(iq.shape[1] // bb)]
+        bb, k = self.cfg.block_bytes, self.cfg.max_blocks
+        n_blocks = iq.shape[1] // bb
+        outs = [self.process(iq[:, b * bb:min(b + k, n_blocks) * bb]) for b in range(0, n_blocks, k)]
         if not outs:
             return np.empty((self.cfg.n_streams, 0), dtype=np.int16)
         return np.concatenate(outs, axis=1)
@@ -169,7 +193,8 @@ class FmBatch:
         L.check(self._lib.fmb_debug_enable(self._h, int(on)), "fmb_debug_enable")
 
     def debug_read(self):
-        n_dem = self.cfg.block_bytes // 16
+        """Discriminator and decoder outputs of the last call (its whole rows)."""
+        n_dem = self._last_blocks * self.cfg.block_bytes // 16
         dem = np.empty((self.cfg.n_streams, n_dem), dtype=np.float32)
         lr = np.empty((self.cfg.n_streams, max(self.max_out, 1)), dtype=np.float32)
         L.check(self._lib.fmb_debug_read(self._h, dem.ctypes.data, n_dem, lr.ctypes.data, lr.shape[1]), "fmb_debug_read")
@@ -195,9 +220,11 @@ class FmBatch:
 
     # -- helpers --------------------------------------------------------------------------------
     def _check_iq(self, iq: np.ndarray) -> np.ndarray:
-        if iq.dtype != np.uint8 or iq.ndim != 2 or iq.shape != (self.cfg.n_streams, self.cfg.block_bytes):
-            raise ValueError(f"iq must be uint8 [{self.cfg.n_streams}, {self.cfg.block_bytes}], got {iq.dtype} {iq.shape}")
-        if iq.strides[1] != 1 or (iq.shape[0] > 1 and (iq.strides[0] < self.cfg.block_bytes or iq.strides[0] % 16)) or iq.ctypes.data % 16:
+        row = self._blocks * self.cfg.block_bytes
+        if iq.dtype != np.uint8 or iq.ndim != 2 or iq.shape != (self.cfg.n_streams, row):
+            raise ValueError(f"iq must be uint8 [{self.cfg.n_streams}, m * {self.cfg.block_bytes}] with "
+                             f"1 <= m <= {self.cfg.max_blocks}, got {iq.dtype} {iq.shape}")
+        if iq.strides[1] != 1 or (iq.shape[0] > 1 and (iq.strides[0] < row or iq.strides[0] % 16)) or iq.ctypes.data % 16:
             iq = np.ascontiguousarray(iq)       # (also a 1-stream view made with iq[None, ...] has stride 0)
             if iq.ctypes.data % 16:
                 buf = np.empty(iq.size + 16, dtype=np.uint8)

@@ -4,7 +4,7 @@
  * branch of output_thread_fn :955-1005), in plain C on top of the C ABI:
  *
  *   one capture file per FM channel  --filesrc_read_async (one thread per channel, 262144-byte chunks)-->
- *   pinned batch buffer [channel][block]  --fmb_multi_submit / fmb_multi_wait (per device: H2D, CUDA kernels, D2H)-->
+ *   pinned batch buffer [channel][K blocks]  --fmb_multi_submit / fmb_multi_wait (per device: H2D, CUDA kernels, D2H)-->
  *   per-channel PCM  --fm_wav (reference WAV header + 32768-byte clusters) or raw .pcm-->
  *
  * The channels are sharded by index over the devices given with -d (default: device 0), one worker thread per
@@ -33,7 +33,7 @@ struct chan {
     int index;
     filesrc_dev_t *src;
     pthread_t thread;
-    long produced;      /* blocks copied into the batch buffers */
+    long produced;      /* blocks copied into the batch buffers (block b goes to step b / K, row slot b % K) */
     int finished;       /* file ended */
     long n_blocks;      /* blocks this channel delivered in total (valid once finished) */
     fm_wav *wav;
@@ -43,11 +43,14 @@ struct chan {
 struct player {
     fmb_config cfg;
     int n;
+    int K;                  /* blocks per channel per step (-K) */
+    size_t row;             /* K * block_bytes */
     struct chan *ch;
-    uint8_t *iq[NBUF];      /* pinned [n][block_bytes] */
+    uint8_t *iq[NBUF];      /* pinned [n][K * block_bytes] */
     int16_t *pcm[NBUF];     /* pinned [n][pcm_pitch]   */
+    int *prefix[NBUF];      /* [K + 1]: int16 values per channel of the first j blocks of the step in that buffer */
     size_t pcm_pitch;
-    long consumed;          /* blocks whose buffers may be refilled: block k may be written iff k < consumed + NBUF */
+    long consumed;          /* steps whose buffers may be refilled: step k may be written iff k < consumed + NBUF */
     pthread_mutex_t mu;
     pthread_cond_t cv;
 };
@@ -65,10 +68,12 @@ static void chunk_cb(unsigned char *buf, uint32_t len, void *ctx)
 {
     struct chan *c = ctx;
     struct player *p = c->p;
+    const long step = c->produced / p->K;
     pthread_mutex_lock(&p->mu);
-    while (c->produced >= p->consumed + NBUF) pthread_cond_wait(&p->cv, &p->mu);
+    while (step >= p->consumed + NBUF) pthread_cond_wait(&p->cv, &p->mu);
     pthread_mutex_unlock(&p->mu);
-    memcpy(p->iq[c->produced % NBUF] + (size_t) c->index * (size_t) p->cfg.block_bytes, buf, len);
+    memcpy(p->iq[step % NBUF] + (size_t) c->index * p->row + (size_t) (c->produced % p->K) * (size_t) p->cfg.block_bytes,
+           buf, len);
     pthread_mutex_lock(&p->mu);
     c->produced++;
     pthread_cond_broadcast(&p->cv);
@@ -94,11 +99,14 @@ static void usage(void)
     fprintf(stderr,
             "fmb_player -- batched offline FM demodulator (B200), one rtl_sdr-format uint8 IQ capture per channel\n"
             "usage: fmb_player [-X | -Y] [-s rate_in] [-r rate_out2] [-E offset] [-m lpr_mode] [-z lpr_size]\n"
-            "                  [-v volume] [-w] [-o out_dir] [-d cuda_devices] [-P exact|fma] [-R speed] capture.u8 ...\n"
+            "                  [-v volume] [-w] [-o out_dir] [-d cuda_devices] [-P exact|fma] [-R speed] [-K blocks]\n"
+            "                  capture.u8 ...\n"
             "  -X  stereo preset 192k/48k, 90 taps   -Y  mono preset 192k/48k, 128 taps   (as rtl_fm_player)\n"
             "  -w  write <name>.wav with the reference's header and 32768-byte cluster rule (default: raw <name>.pcm)\n"
             "  -d  CUDA devices to shard the channels over, e.g. 0-7 or 0,2,4 (default 0); at least one channel per device\n"
-            "  -R  pace the captures at `speed` x real time (default: as fast as the GPU takes them)\n");
+            "  -R  pace the captures at `speed` x real time (default: as fast as the GPU takes them)\n"
+            "  -K  consecutive 262144-byte blocks of every channel per GPU step (default 1): fewer, larger steps fill the\n"
+            "      GPU when there are few channels; the output is the same\n");
 }
 
 static const char *base_name(const char *path)
@@ -120,6 +128,7 @@ int main(int argc, char **argv)
     fmb_multi *h = NULL;
 
     memset(&P, 0, sizeof P);
+    P.K = 1;
     devices[0] = 0;
     fmb_default_config(&P.cfg);
     for (i = 1; i < argc; ++i) {
@@ -139,14 +148,18 @@ int main(int argc, char **argv)
         else if (!strcmp(a, "-o") && i + 1 < argc) out_dir = argv[++i];
         else if (!strcmp(a, "-R") && i + 1 < argc) speed = atof(argv[++i]);
         else if (!strcmp(a, "-P") && i + 1 < argc) P.cfg.precision = !strcmp(argv[++i], "fma") ? FMB_PRECISION_FMA : FMB_PRECISION_EXACT;
+        else if (!strcmp(a, "-K") && i + 1 < argc) P.K = atoi(argv[++i]);
         else if (!strcmp(a, "-w")) wav = 1;
         else if (!strcmp(a, "-h")) { usage(); return 0; }
         else if (a[0] == '-' && a[1]) { usage(); return 2; }
         else { first_file = i; break; }
     }
     if (first_file < 0) { usage(); return 2; }
+    if (P.K < 1) { fprintf(stderr, "-K: need at least one block per step\n"); return 2; }
     P.n = argc - first_file;
     P.cfg.n_streams = P.n;
+    P.cfg.max_blocks_per_call = P.K;
+    P.row = (size_t) P.K * (size_t) P.cfg.block_bytes;
     P.ch = calloc((size_t) P.n, sizeof *P.ch);
     n_outs = calloc((size_t) P.n, sizeof *n_outs);
     if (!P.ch || !n_outs) return 1;
@@ -159,11 +172,13 @@ int main(int argc, char **argv)
     if (rc != FMB_OK) { fprintf(stderr, "fmb_multi_create: %s\n", fmb_last_error()); return 1; }
     P.pcm_pitch = ((size_t) fmb_multi_max_out_count(h) + 7) & ~(size_t) 7;
     for (i = 0; i < NBUF; ++i) {
-        if (fmb_host_alloc((void **) &P.iq[i], (size_t) P.n * (size_t) P.cfg.block_bytes) != FMB_OK ||
+        if (fmb_host_alloc((void **) &P.iq[i], (size_t) P.n * P.row) != FMB_OK ||
             fmb_host_alloc((void **) &P.pcm[i], (size_t) P.n * P.pcm_pitch * sizeof(int16_t)) != FMB_OK) {
             fprintf(stderr, "pinned allocation: %s\n", fmb_last_error());
             return 1;
         }
+        P.prefix[i] = calloc((size_t) P.K + 1, sizeof(int));
+        if (!P.prefix[i]) return 1;
     }
     for (i = 0; i < P.n; ++i) {
         struct chan *c = &P.ch[i];
@@ -181,42 +196,52 @@ int main(int argc, char **argv)
     t0 = now_s();
     for (i = 0; i < P.n; ++i) pthread_create(&P.ch[i].thread, NULL, reader, &P.ch[i]);
 
-    /* the demod thread of this program: block k of every channel -> one fmb_submit */
+    /* the demod thread of this program: blocks [k*K, (k+1)*K) of every channel -> one fmb_submit */
     for (k = 0;; ++k) {
-        int live = 0, n_out = 0;
+        int live = 0;
         pthread_mutex_lock(&P.mu);
-        for (;;) { /* wait until every channel has either delivered block k or ended */
+        for (;;) { /* wait until every channel has either delivered the blocks of step k or ended */
             int ready = 1;
             live = 0;
             for (i = 0; i < P.n; ++i) {
-                if (P.ch[i].produced > k) live++;
-                else if (!P.ch[i].finished) ready = 0;
+                if (P.ch[i].produced > k * P.K) live++;
+                if (P.ch[i].produced < (k + 1) * P.K && !P.ch[i].finished) ready = 0;
             }
             if (ready) break;
             pthread_cond_wait(&P.cv, &P.mu);
         }
         pthread_mutex_unlock(&P.mu);
         if (live > 0) {
-            for (i = 0; i < P.n; ++i) /* ended channels get mid-scale bytes; their PCM is not written */
-                if (P.ch[i].produced <= k) memset(P.iq[k % NBUF] + (size_t) i * (size_t) P.cfg.block_bytes, 127, (size_t) P.cfg.block_bytes);
-            rc = fmb_multi_submit(h, P.iq[k % NBUF], (size_t) P.cfg.block_bytes, P.pcm[k % NBUF], P.pcm_pitch, &tickets[k % NBUF]);
+            int j;
+            for (i = 0; i < P.n; ++i) { /* rows of ended channels get mid-scale bytes; their PCM is not written */
+                const long have = P.ch[i].produced - k * P.K;
+                if (have < P.K) {
+                    const size_t from = have > 0 ? (size_t) have * (size_t) P.cfg.block_bytes : 0;
+                    memset(P.iq[k % NBUF] + (size_t) i * P.row + from, 127, P.row - from);
+                }
+            }
+            for (j = 0; j <= P.K; ++j) P.prefix[k % NBUF][j] = fmb_multi_out_count_blocks(h, j);
+            rc = fmb_multi_submit(h, P.iq[k % NBUF], P.row, P.pcm[k % NBUF], P.pcm_pitch, &tickets[k % NBUF]);
             if (rc != FMB_OK) { fprintf(stderr, "fmb_multi_submit: %s\n", fmb_last_error()); return 1; }
             submitted = k + 1;
         }
-        /* retire block k-(NBUF-1) (or everything left once the inputs have ended) */
+        /* retire step k-(NBUF-1) (or everything left once the inputs have ended) */
         {
             long upto = live > 0 ? submitted - (NBUF - 1) : submitted, j;
             for (j = P.consumed; j < upto; ++j) {
-                rc = fmb_multi_wait(h, tickets[j % NBUF], n_outs);   /* result_len of this block, per channel */
+                rc = fmb_multi_wait(h, tickets[j % NBUF], n_outs);   /* result_len of the step's blocks, per channel */
                 if (rc != FMB_OK) { fprintf(stderr, "fmb_multi_wait: %s\n", fmb_last_error()); return 1; }
-                n_out = n_outs[0];
                 for (i = 0; i < P.n; ++i) {
                     struct chan *c = &P.ch[i];
                     const int16_t *src = P.pcm[j % NBUF] + (size_t) i * P.pcm_pitch;
-                    if (c->finished && j >= c->n_blocks) continue;
+                    long blocks = P.K;                       /* of this channel in step j */
+                    int n_out;
+                    if (c->finished && c->n_blocks - j * P.K < blocks) blocks = c->n_blocks - j * P.K;
+                    if (blocks <= 0) continue;
+                    n_out = P.prefix[j % NBUF][blocks];      /* the PCM of its first `blocks` blocks */
                     if (c->wav) fm_wav_write(c->wav, src, (size_t) n_out * 2);
                     else fwrite(src, 2, (size_t) n_out, c->raw);
-                    total_blocks++;
+                    total_blocks += blocks;
                 }
                 pthread_mutex_lock(&P.mu);
                 P.consumed = j + 1;
@@ -238,7 +263,7 @@ int main(int argc, char **argv)
         if (P.ch[i].raw) fclose(P.ch[i].raw);
         filesrc_close(P.ch[i].src);
     }
-    for (i = 0; i < NBUF; ++i) { fmb_host_free(P.iq[i]); fmb_host_free(P.pcm[i]); }
+    for (i = 0; i < NBUF; ++i) { fmb_host_free(P.iq[i]); fmb_host_free(P.pcm[i]); free(P.prefix[i]); }
     fmb_multi_destroy(h);
     free(P.ch);
     free(n_outs);

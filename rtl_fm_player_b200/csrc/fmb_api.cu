@@ -53,7 +53,7 @@ struct Slot { /* one in-flight block-step of the pipelined host path */
     uint8_t *d_iq = nullptr;
     int16_t *d_pcm = nullptr;
     cudaEvent_t ev_h2d = nullptr, ev_iq_free = nullptr, ev_done = nullptr;
-    int n_out = 0;
+    int n_out = 0;                 /* of this submit's blocks */
     bool busy = false;
 };
 
@@ -62,16 +62,23 @@ struct Slot { /* one in-flight block-step of the pipelined host path */
 struct fmb_handle {
     fmb_config cfg;
     fmb_tables tab;
-    int n_dem;                 /* demodulated samples per stream per step */
-    /* launch geometry and work-assignment policy of one demod kernel */
+    int n_dem;                 /* demodulated samples per stream per block */
+    int max_blocks = 1;        /* cfg.max_blocks_per_call (0 -> 1): blocks per stream per call, at most */
+    int blocks = 1;            /* ... in the next call (fmb_set_blocks_per_call) */
+    /* launch geometry and work-assignment policy of one demod kernel, for a call of a given number of blocks */
     struct Plan {
         int grid = 0;              /* CTAs */
         int ctas_per_sm = 0;       /* > 0 when the grid is exactly one full wave (SMs x occupancy) */
         int chunk = 0, n_whole = 0; /* dynamic work assignment (0 = static), see fmb_kparams */
     };
-    Plan plan;                 /* fmb_demod_kernel */
-    Plan plan_ws;              /* the warp-specialised kernel of this configuration (grid 0: none) */
+    int sms = 0;               /* multiprocessors of cfg.device */
+    int occ = 0, occ_ws = 0;   /* resident CTAs per SM of fmb_demod_kernel / the warp-specialised kernel (0: none) */
+    int env_chunk = -1, env_tail = -1; /* FMB_CHUNK / FMB_TAIL_PCT as read at create (-1: not set) */
     bool ws_generic = true;    /* ... also off the 4:1 fast path (env FMB_WS_GENERIC=0: A/B) */
+    int de_warps = 0;          /* de-emphasis warps the device holds at once (sizes the time segments of long rows) */
+    float *d_seg_state = nullptr; /* [stream][segments][4] de-emphasis segment junctions (max_blocks > 1 only) */
+    unsigned int *d_seg_count = nullptr; /* [stream] segments finished in the running pass (max_blocks > 1 only) */
+    int max_segs = 1;
     unsigned int *d_tickets = nullptr;         /* FMB_TICKET_SLOTS counters, used in rotation by launch sequence number */
     unsigned int ticket_base[FMB_TICKET_SLOTS] = {};
     /* overlap of consecutive demod launches (programmatic dependent launch, see fmb_kparams.done) */
@@ -98,7 +105,7 @@ struct fmb_handle {
     int lr_cur = 0;
     float *d_dem = nullptr;          /* debug tap */
     int debug = 0;
-    int last_n_out = 0, last_lr = 0;
+    int last_n_out = 0, last_lr = 0, last_blocks = 1;
     int fast = 0;                    /* the resampler's fast rate: cfg.rate_out, or rate_in when that is 0 (:485) */
     /* the caller stream of the previous step: when it changes, the new stream first waits for that step's demod
      * kernel (it wrote the carried state and drew from the ticket counter this step continues from) */
@@ -110,6 +117,7 @@ struct fmb_handle {
     cudaStream_t s_aux = nullptr, s_main = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_demod[kLrBufs] = {}, ev_deemph[kLrBufs] = {};
     bool deemph_pending[kLrBufs] = {};
+    bool deemph_segmented[kLrBufs] = {};  /* that pass was fmb_deemph_seg_kernel (a row of several blocks) */
     cudaEvent_t ev_fork = nullptr;
     /* pipelined host path */
     Slot slot[FMB_PIPE_DEPTH];
@@ -125,20 +133,20 @@ struct fmb_handle {
 
 namespace {
 
-/* int16 values the step starting at resampler phase `phase` produces */
-int out_count_for(const fmb_handle *h, int phase)
+/* int16 values the first n blocks of a step starting at resampler phase `phase` produce */
+int out_count_for(const fmb_handle *h, int phase, int n = 1)
 {
     const fmb_config &c = h->cfg;
-    if (c.rate_out2 <= 0) return h->n_dem;
-    const long long ticks = ((long long) phase + (long long) h->n_dem * c.rate_out2) / h->fast;
+    if (c.rate_out2 <= 0) return n * h->n_dem;
+    const long long ticks = ((long long) phase + (long long) n * h->n_dem * c.rate_out2) / h->fast;
     return (int) (c.mode == 2 ? 2 * ticks : ticks);
 }
 
-int next_phase(const fmb_handle *h, int phase)
+int next_phase(const fmb_handle *h, int phase, int n = 1)
 {
     const fmb_config &c = h->cfg;
     if (c.rate_out2 <= 0) return phase;
-    return (int) (((long long) phase + (long long) h->n_dem * c.rate_out2) % h->fast);
+    return (int) (((long long) phase + (long long) n * h->n_dem * c.rate_out2) % h->fast);
 }
 
 /* Does the reference's in-place output overwrite (src/rtl_fm_player.c:593-597)
@@ -196,12 +204,6 @@ int check_inplace_cycle(const fmb_handle *h, int phase0)
     return FMB_OK;
 }
 
-bool tick_on_first_sample(const fmb_handle *h, int phase)
-{
-    const fmb_config &c = h->cfg;
-    return c.mode == 2 && c.rate_out2 > 0 && (long long) phase + c.rate_out2 >= h->fast;
-}
-
 void destroy_events(cudaEvent_t *ev, int n)
 {
     if (!ev) return;
@@ -253,10 +255,102 @@ int check_device_error(fmb_handle *h)
 bool ws_kernel_applies(const fmb_handle *h, bool dec4)
 {
     /* mono: the 4:1 fast path and any other ratio on the kernel's generic tick path (FMB_WS_GENERIC=0: fast path only) */
-    return h->plan_ws.grid > 0 && (dec4 || h->ws_generic) && h->cfg.mode == 1 && h->cfg.rate_out2 > 0;
+    return h->occ_ws > 0 && (dec4 || h->ws_generic) && h->cfg.mode == 1 && h->cfg.rate_out2 > 0;
 }
 
-/* Enqueue one block-step: demod kernel on `sm`, de-emphasis kernel on the aux
+/* Does a block of the call of n blocks starting at `phase` start with a tick on its sample 0 (the in-place quirk,
+ * SURVEY A.7)?  When none does the kernel is told nothing about blocks (blk_dem 0) and skips the per-step test. */
+bool quirk_in_call(const fmb_handle *h, int phase, int n)
+{
+    const fmb_config &c = h->cfg;
+    if (!c.emulate_inplace_quirk || c.mode != 2 || c.rate_out2 <= 0) return false;
+    for (int b = 0; b < n; ++b, phase = next_phase(h, phase))
+        if ((long long) phase + c.rate_out2 >= h->fast) return true;
+    return false;
+}
+
+/* cudaMalloc that reports an allocation the device cannot satisfy as FMB_ERR_NOMEM (such a failure is not sticky) */
+int dev_alloc(void **p, size_t bytes, const char *what)
+{
+    const cudaError_t e = cudaMalloc(p, bytes);
+    if (e == cudaErrorMemoryAllocation) {
+        cudaGetLastError();
+        *p = nullptr;
+        return set_err(FMB_ERR_NOMEM, what, e);
+    }
+    if (e != cudaSuccess) return set_err(FMB_ERR_CUDA, what, e);
+    return FMB_OK;
+}
+
+/* CTAs and work assignment of a call of n blocks per stream: the n_streams x (n x block/2048 samples) work units are
+ * dealt out evenly ("stream-K").  Default: one CTA per resident slot (SMs x occupancy); cfg.segments > 0 forces
+ * n_streams x segments CTAs per block.
+ * Dynamic work assignment (see fmb_demod_kernel) pays when every CTA of the resident wave has several blocks' worth of
+ * work.  One block per call: whole streams first, and about FMB_DEFAULT_TAIL_RUNS fine-grain runs of FMB_CHUNK
+ * sub-tiles per CTA at the end of the launch, so that the CTAs finish together.  Smaller batches (64 streams on 444
+ * CTAs) keep the static split into equal runs: a whole stream would be several CTAs' share.  Several blocks per call:
+ * tickets of one block each once every CTA has two blocks, else the static split (DESIGN.md "Several blocks per
+ * call").  FMB_CHUNK / FMB_TAIL_PCT (percent of the streams handed out in fine-grain runs) override the policy, for
+ * tuning and tests; FMB_CHUNK=0 forces the static split. */
+fmb_handle::Plan plan_for(const fmb_handle *h, int n, bool ws)
+{
+    const fmb_config &c = h->cfg;
+    fmb_handle::Plan pl;
+    const int occ = ws ? h->occ_ws : h->occ;
+    if (c.segments > 0) {
+        if (!ws) pl.grid = c.n_streams * c.segments * n;
+        return pl;
+    }
+    if (occ <= 0) return pl;
+    const int blk_spb = h->n_dem / FMB_NSUB, spb = n * blk_spb;
+    const long long units = (long long) c.n_streams * spb, slots = (long long) occ * h->sms;
+    pl.grid = (int) (units < slots ? units : slots);
+    if (units < slots) return pl;
+    pl.ctas_per_sm = occ;
+    const bool forced = h->env_chunk >= 0 || h->env_tail >= 0;
+    if (n > 1 && !forced) {
+        if (units >= 2LL * blk_spb * pl.grid) { pl.chunk = blk_spb; pl.n_whole = 0; }
+        return pl;
+    }
+    const int chunk = h->env_chunk >= 0 ? h->env_chunk : FMB_DEFAULT_CHUNK;
+    if (!(chunk > 0 && chunk <= spb && spb % chunk == 0 && (forced || units >= 2LL * spb * pl.grid)))
+        return pl;
+    int tail_streams;
+    if (h->env_tail >= 0) {
+        int tail = h->env_tail;
+        tail = tail < 0 ? 0 : tail > 100 ? 100 : tail;
+        tail_streams = c.n_streams - (int) ((long long) c.n_streams * (100 - tail) / 100);
+    } else if (h->pdl) {
+        /* overlapping launches: the CTAs of the next launch take over the slots this launch's ragged end
+         * frees, so nothing has to finish together -- every stream is handed out whole (no lead-ins to
+         * recompute).  1024 streams: 0.3475 -> 0.3337 ms per step (profiles/r02g_pdl_tail_sweep.txt) */
+        tail_streams = 0;
+    } else {
+        tail_streams = (FMB_DEFAULT_TAIL_RUNS * chunk * pl.grid + spb - 1) / spb;
+        if (tail_streams > c.n_streams) tail_streams = c.n_streams;
+    }
+    pl.chunk = chunk;
+    pl.n_whole = c.n_streams - tail_streams;
+    return pl;
+}
+
+/* Time segments per stream of the de-emphasis of a row of n_out values: enough warps to fill the device, segments of
+ * at least FMB_DE_MIN_SEG_CHUNKS chunks, and a one-block row always in one piece (fmb_deemph_kernel). */
+void deemph_segments(const fmb_handle *h, int n_blocks, int n_out, int *segs, int *seg_chunks)
+{
+    *segs = 1; *seg_chunks = 0;
+    if (n_blocks <= 1 || !h->d_seg_state) return;
+    const long long n_chunk = (n_out + FMB_DE_CHUNK - 1) / FMB_DE_CHUNK;
+    long long s = (h->de_warps + h->cfg.n_streams - 1) / h->cfg.n_streams;
+    if (s > n_chunk / FMB_DE_MIN_SEG_CHUNKS) s = n_chunk / FMB_DE_MIN_SEG_CHUNKS;
+    if (s > h->max_segs) s = h->max_segs;
+    if (s <= 1) return;
+    const long long per = (n_chunk + s - 1) / s;
+    *seg_chunks = (int) per;
+    *segs = (int) ((n_chunk + per - 1) / per);
+}
+
+/* Enqueue one step of h->blocks blocks: demod kernel on `sm`, de-emphasis kernel(s) on the aux
  * stream.  d_iq/d_pcm are device pointers. */
 int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d_pcm, size_t pcm_pitch,
                  cudaStream_t sm, int *n_out_ret)
@@ -264,12 +358,13 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     const fmb_config &c = h->cfg;
     if (h->poisoned)
         return set_err(FMB_ERR_STATE, "an earlier CUDA failure left this handle half-advanced; fmb_reset() or destroy it");
-    const int n_out = out_count_for(h, h->phase);
+    const int nb = h->blocks;
+    const int n_out = out_count_for(h, h->phase, nb);
     if ((size_t) n_out > pcm_pitch) return set_err(FMB_ERR_ARG, "pcm_pitch smaller than fmb_next_out_count()");
-    if (iq_pitch < (size_t) c.block_bytes || (iq_pitch & 15) || ((uintptr_t) d_iq & 15))
-        return set_err(FMB_ERR_ARG, "iq pointer/pitch must be 16-byte aligned and pitch >= block_bytes");
-    const bool quirk = c.emulate_inplace_quirk && tick_on_first_sample(h, h->phase);
-    if (c.emulate_inplace_quirk && inplace_hazard(h, h->phase))   /* refused at create/set_state; cheap re-check */
+    if (iq_pitch < (size_t) nb * c.block_bytes || (iq_pitch & 15) || ((uintptr_t) d_iq & 15))
+        return set_err(FMB_ERR_ARG, "iq pointer/pitch must be 16-byte aligned and pitch >= blocks per call x block_bytes");
+    /* refused at create/set_state; cheap re-check (the call's later blocks start at phases of the same cycle) */
+    if (c.emulate_inplace_quirk && inplace_hazard(h, h->phase))
         return set_err(FMB_ERR_UNSUPPORTED, "in-place stereo output would overwrite unread input (see fmb_create)");
 
     const int b = h->lr_cur;
@@ -281,7 +376,11 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
      * launch overwrites it.  With overlapping launches that is ordered per stream inside the kernel (de_done, see
      * wait_stream) and NO stream operation is put between this launch and the previous one -- a cross-stream wait
      * here would serialise them again.  Without overlap the event does it. */
-    if (h->deemph_pending[b] && !h->pdl) CU(cudaStreamWaitEvent(sm, h->ev_deemph[b], 0));
+    /* A pass over a row of several blocks is no shorter than a demod launch of few streams and has as many CTAs: it
+     * would not get its SM slots back from overlapping CTAs that wait for it in the kernel (measured: a hand-over
+     * time-out at 8 mono streams x 16 blocks).  Such a pass is waited for here, and this launch does not overlap. */
+    const bool wait_deemph = h->deemph_pending[b] && (!h->pdl || h->deemph_segmented[b]);
+    if (wait_deemph) CU(cudaStreamWaitEvent(sm, h->ev_deemph[b], 0));
 
     fmb_kparams kp;
     memset(&kp, 0, sizeof kp);
@@ -292,16 +391,16 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     kp.lr = h->d_lr[b];
     kp.lr_pitch = h->lr_pitch;
     kp.dem_dump = h->debug ? h->d_dem : nullptr;
-    kp.dem_pitch = h->n_dem;
+    kp.dem_pitch = (long long) h->max_blocks * h->n_dem;
     kp.n_streams = c.n_streams;
     /* which kernel: the warp-specialised one where this configuration has it and the resampler is on its 4:1 fast path */
     const bool dec4 = c.rate_out2 > 0 && h->fast % c.rate_out2 == 0 && h->phase % c.rate_out2 == 0 &&
                       h->fast / c.rate_out2 == 4 && h->phase / c.rate_out2 == 0;
     const bool ws = ws_kernel_applies(h, dec4);
-    const fmb_handle::Plan &pl = ws ? h->plan_ws : h->plan;
+    const fmb_handle::Plan pl = plan_for(h, nb, ws);
     kp.ws = ws ? 1 : 0;
     kp.grid = pl.grid;
-    kp.n_dem = h->n_dem;
+    kp.n_dem = nb * h->n_dem;
     if (c.rate_out2 > 0) {
         kp.slow = c.rate_out2; kp.fast = h->fast; kp.phase0 = h->phase;
         if (h->fast % c.rate_out2 == 0 && h->phase % c.rate_out2 == 0) {
@@ -311,10 +410,10 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     } else { /* lp_real_f32 skipped: every sample is an output */
         kp.slow = 1; kp.fast = 1; kp.phase0 = 0; kp.dec = 1; kp.dec_c0 = 0;
     }
-    kp.quirk = quirk ? 1 : 0;
+    kp.blk_dem = quirk_in_call(h, h->phase, nb) ? h->n_dem : 0;
     unsigned int ticket_step = 0;      /* tickets this launch consumes; committed with the rest of the bookkeeping */
     if (pl.chunk > 0) {
-        const int spb = h->n_dem / FMB_NSUB;
+        const int spb = kp.n_dem / FMB_NSUB;
         kp.chunk = pl.chunk;
         kp.n_whole = pl.n_whole;
         kp.tickets = h->d_tickets + (h->seq % FMB_TICKET_SLOTS);
@@ -326,7 +425,7 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     kp.de_done = h->d_de_done;
     kp.seq = h->seq;
     kp.dev_err = h->d_err;
-    kp.pdl = h->pdl && !h->serial_next;
+    kp.pdl = h->pdl && !h->serial_next && !wait_deemph;
 
     fmb_config kc = c;
     if (c.rate_out2 <= 0) kc.mode = 0;
@@ -362,6 +461,9 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     dp.pcm_scale = h->tab.pcm_scale;
     dp.fallbacks = h->d_fallbacks;
     dp.de_done = h->d_de_done;
+    deemph_segments(h, nb, n_out, &dp.segs, &dp.seg_chunks);
+    dp.seg_state = h->d_seg_state;
+    dp.seg_count = h->d_seg_count;
     if (prof) CUP(cudaEventRecord(h->pev[1][0][h->pcount[1]], h->s_aux));
 #ifdef FMB_TUNE_SKIP_DEEMPH   /* tools/build_variant.sh only: timing experiment, PCM is not produced */
     e = cudaSuccess;
@@ -374,6 +476,7 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     CUP(cudaEventRecord(h->ev_deemph[b], h->s_aux));
 #undef CUP
     h->deemph_pending[b] = true;
+    h->deemph_segmented[b] = dp.segs > 1;
     h->ticket_base[h->seq % FMB_TICKET_SLOTS] += ticket_step;
     h->seq++;
     h->serial_next = false;
@@ -381,11 +484,12 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     h->have_last_stream = true;
 
     h->last_n_out = n_out;
+    h->last_blocks = nb;
     h->last_lr = b;
     h->lr_cur = (h->lr_cur + 1) % kLrBufs;
     h->state_cur ^= 1;
-    h->phase = next_phase(h, h->phase);
-    h->blocks_done++;
+    h->phase = next_phase(h, h->phase, nb);
+    h->blocks_done += (uint64_t) nb;
     if (n_out_ret) *n_out_ret = n_out;
     return FMB_OK;
 }
@@ -452,6 +556,10 @@ int fmb_create(const fmb_config *cfg, fmb_handle **out)
     if (cfg->precision != FMB_PRECISION_EXACT && cfg->precision != FMB_PRECISION_FMA)
         return set_err(FMB_ERR_ARG, "bad precision");
     if (cfg->rate_out < 0) return set_err(FMB_ERR_ARG, "bad rate_out");
+    /* the kernels address a stream's row of one call with int sample and byte offsets */
+    if (cfg->max_blocks_per_call < 0 ||
+        (long long) (cfg->max_blocks_per_call > 0 ? cfg->max_blocks_per_call : 1) * cfg->block_bytes >= (1LL << 31))
+        return set_err(FMB_ERR_ARG, "max_blocks_per_call must be >= 0 and max_blocks_per_call * block_bytes < 2^31");
     const int fast = cfg->rate_out > 0 ? cfg->rate_out : cfg->rate_in;
     if (cfg->rate_out2 > fast) return set_err(FMB_ERR_UNSUPPORTED, "rate_out2 > rate_out");
     /* the tick schedule of a sub-tile is evaluated in 32-bit arithmetic: (ticks + 1) * rate_out must fit */
@@ -478,67 +586,72 @@ int fmb_create(const fmb_config *cfg, fmb_handle **out)
     int rc = fmb_design_tables(cfg, &h->tab);
     if (rc != FMB_OK) { delete h; return set_err(rc, "filter design rejected the configuration"); }
     h->n_dem = cfg->block_bytes / 16;
+    h->max_blocks = cfg->max_blocks_per_call > 0 ? cfg->max_blocks_per_call : 1;
+    h->blocks = h->max_blocks;
     h->fast = fast;
     rc = check_inplace_cycle(h, 0);
     if (rc != FMB_OK) { delete h; return rc; }
+    if (cfg->segments > 0 && (h->n_dem / FMB_NSUB) % cfg->segments) {
+        delete h;
+        return set_err(FMB_ERR_ARG, "segments must divide block_bytes/32768");
+    }
     {
-        /* CTAs: the n_streams x (block/2048 samples) work units are dealt out evenly ("stream-K").
-         * Default: one CTA per resident slot (SMs x occupancy); cfg.segments > 0 forces n_streams x segments. */
-        const long long units = (long long) cfg->n_streams * (h->n_dem / FMB_NSUB);
-        if (cfg->segments > 0) {
-            if ((h->n_dem / FMB_NSUB) % cfg->segments) {
-                delete h;
-                return set_err(FMB_ERR_ARG, "segments must divide block_bytes/32768");
-            }
-            h->plan.grid = cfg->n_streams * cfg->segments;
-        } else {
-            fmb_config kc = *cfg;
-            if (cfg->rate_out2 <= 0) kc.mode = 0;
-            int occ = 0, occ_ws = 0, sms = 0;
-            cudaError_t e1 = (cudaError_t) fmb_demod_occupancy(&kc, &occ);
-            cudaError_t e2 = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
-            if (e1 != cudaSuccess || e2 != cudaSuccess || occ < 1 || sms < 1) {
-                delete h;
-                return set_err(FMB_ERR_CUDA, "occupancy query for the demod kernel", e1 != cudaSuccess ? e1 : e2);
-            }
-            {
-                /* FMB_MAX_CTAS_PER_SM: run with fewer resident CTAs per SM than fit (diagnostic: how the step time
-                 * scales with the number of CTAs that share an SM) */
-                const char *em = getenv("FMB_MAX_CTAS_PER_SM");
-                if (em && atoi(em) > 0 && atoi(em) < occ) occ = atoi(em);
-            }
-            const long long slots = (long long) occ * sms;
-            h->plan.grid = (int) (units < slots ? units : slots);
-            if (units >= slots) h->plan.ctas_per_sm = occ;
-            /* FMB_WS=0: never use the warp-specialised kernels (tuning / A-B comparison) */
-            const char *ew = getenv("FMB_WS");
-            const char *eg = getenv("FMB_WS_GENERIC");
-            h->ws_generic = !(eg && atoi(eg) == 0);
-            if (!(ew && atoi(ew) == 0) && cfg->rate_out2 > 0) {
-                e1 = (cudaError_t) fmb_demod_ws_occupancy(&kc, &occ_ws);
-                if (e1 != cudaSuccess) { delete h; return set_err(FMB_ERR_CUDA, "occupancy query for the warp-specialised kernel", e1); }
-                {
-                    const char *em = getenv("FMB_MAX_CTAS_PER_SM");
-                    if (em && atoi(em) > 0 && atoi(em) < occ_ws) occ_ws = atoi(em);
-                }
-                if (occ_ws > 0) {
-                    const long long slots_ws = (long long) occ_ws * sms;
-                    h->plan_ws.grid = (int) (units < slots_ws ? units : slots_ws);
-                    if (units >= slots_ws) h->plan_ws.ctas_per_sm = occ_ws;
-                }
-            }
+        int warps = 0;
+        cudaError_t e1 = cudaDeviceGetAttribute(&h->sms, cudaDevAttrMultiProcessorCount, cfg->device);
+        cudaError_t e2 = (cudaError_t) fmb_deemph_occupancy(&warps);
+        if (e1 != cudaSuccess || e2 != cudaSuccess || h->sms < 1) {
+            delete h;
+            return set_err(FMB_ERR_CUDA, "device attribute / de-emphasis occupancy query", e1 != cudaSuccess ? e1 : e2);
         }
+        h->de_warps = warps * h->sms;
+    }
+    if (cfg->segments <= 0) {
+        /* resident CTAs per SM of the kernels this configuration may launch; the launch plan of each call
+         * follows from them (plan_for) */
+        fmb_config kc = *cfg;
+        if (cfg->rate_out2 <= 0) kc.mode = 0;
+        int occ = 0, occ_ws = 0;
+        cudaError_t e1 = (cudaError_t) fmb_demod_occupancy(&kc, &occ);
+        if (e1 != cudaSuccess || occ < 1) {
+            delete h;
+            return set_err(FMB_ERR_CUDA, "occupancy query for the demod kernel", e1);
+        }
+        /* FMB_MAX_CTAS_PER_SM: run with fewer resident CTAs per SM than fit (diagnostic: how the step time
+         * scales with the number of CTAs that share an SM) */
+        const char *em = getenv("FMB_MAX_CTAS_PER_SM");
+        if (em && atoi(em) > 0 && atoi(em) < occ) occ = atoi(em);
+        h->occ = occ;
+        /* FMB_WS=0: never use the warp-specialised kernels (tuning / A-B comparison) */
+        const char *ew = getenv("FMB_WS");
+        const char *eg = getenv("FMB_WS_GENERIC");
+        h->ws_generic = !(eg && atoi(eg) == 0);
+        if (!(ew && atoi(ew) == 0) && cfg->rate_out2 > 0) {
+            e1 = (cudaError_t) fmb_demod_ws_occupancy(&kc, &occ_ws);
+            if (e1 != cudaSuccess) { delete h; return set_err(FMB_ERR_CUDA, "occupancy query for the warp-specialised kernel", e1); }
+            if (em && atoi(em) > 0 && atoi(em) < occ_ws) occ_ws = atoi(em);
+            h->occ_ws = occ_ws;
+        }
+    }
+    {
+        const char *ec = getenv("FMB_CHUNK"), *et = getenv("FMB_TAIL_PCT");
+        h->env_chunk = ec ? (atoi(ec) > 0 ? atoi(ec) : 0) : -1;
+        h->env_tail = et ? (atoi(et) > 0 ? atoi(et) : 0) : -1;
     }
     h->phase = 0;
     h->blocks_done = 0;
-    /* upper bound of outputs per step */
+    /* upper bound of outputs per step (at the most blocks per call) */
+    const long long max_dem = (long long) h->max_blocks * h->n_dem;
     if (cfg->rate_out2 > 0) {
-        const long long t = ((long long) fast - 1 + (long long) h->n_dem * cfg->rate_out2) / fast;
+        const long long t = ((long long) fast - 1 + max_dem * cfg->rate_out2) / fast;
         h->max_out = (int) (cfg->mode == 2 ? 2 * t : t);
     } else {
-        h->max_out = h->n_dem;
+        h->max_out = (int) max_dem;
     }
     h->lr_pitch = ((long long) h->max_out + 127) & ~127LL; /* whole de-emphasis stages */
+    if (h->max_blocks > 1) {
+        const long long m = ((h->max_out + FMB_DE_CHUNK - 1) / FMB_DE_CHUNK) / FMB_DE_MIN_SEG_CHUNKS;
+        h->max_segs = m > 1 ? (int) m : 1;
+    }
 
     const size_t st_bytes = sizeof(fmb_stream_state) * (size_t) cfg->n_streams;
 #define CUH(call)                                                                                   \
@@ -546,16 +659,28 @@ int fmb_create(const fmb_config *cfg, fmb_handle **out)
         cudaError_t e_ = (call);                                                                    \
         if (e_ != cudaSuccess) { set_err(FMB_ERR_CUDA, #call, e_); fmb_destroy(h); return FMB_ERR_CUDA; } \
     } while (0)
+    /* buffers whose size grows with max_blocks_per_call: a size that does not fit is FMB_ERR_NOMEM */
+#define CUA(ptr, bytes)                                                                             \
+    do {                                                                                            \
+        const int rc_ = dev_alloc((void **) &(ptr), (bytes), #ptr);                                 \
+        if (rc_ != FMB_OK) { fmb_destroy(h); return rc_; }                                          \
+    } while (0)
     for (int i = 0; i < 2; ++i) {
         CUH(cudaMalloc(&h->d_state[i], st_bytes));
         CUH(cudaMemset(h->d_state[i], 0, st_bytes));
     }
     for (int i = 0; i < kLrBufs; ++i) {
-        CUH(cudaMalloc(&h->d_lr[i], (size_t) h->lr_pitch * cfg->n_streams * sizeof(float)));
+        CUA(h->d_lr[i], (size_t) h->lr_pitch * cfg->n_streams * sizeof(float));
         CUH(cudaMemset(h->d_lr[i], 0, (size_t) h->lr_pitch * cfg->n_streams * sizeof(float)));
         CUH(cudaEventCreateWithFlags(&h->ev_demod[i], cudaEventDisableTiming));
         CUH(cudaEventCreateWithFlags(&h->ev_deemph[i], cudaEventDisableTiming));
     }
+    if (h->max_blocks > 1) {
+        CUA(h->d_seg_state, sizeof(float) * 4 * (size_t) h->max_segs * cfg->n_streams);
+        CUA(h->d_seg_count, sizeof(unsigned int) * (size_t) cfg->n_streams);
+        CUH(cudaMemset(h->d_seg_count, 0, sizeof(unsigned int) * (size_t) cfg->n_streams));
+    }
+#undef CUA
     CUH(cudaMalloc(&h->d_de_state, sizeof(float) * 2 * (size_t) cfg->n_streams));
     CUH(cudaMemset(h->d_de_state, 0, sizeof(float) * 2 * (size_t) cfg->n_streams));
     CUH(cudaMalloc(&h->d_fallbacks, sizeof(unsigned int)));
@@ -574,40 +699,6 @@ int fmb_create(const fmb_config *cfg, fmb_handle **out)
         /* FMB_PDL=0: plain stream order between consecutive demod launches (tuning / A-B comparison) */
         const char *ep = getenv("FMB_PDL");
         h->pdl = (ep && atoi(ep) == 0) ? 0 : 1;
-    }
-    {
-        /* Dynamic work assignment (see fmb_demod_kernel).  It pays when every CTA of the resident wave has
-         * several streams' worth of work: whole streams first, and about FMB_DEFAULT_TAIL_RUNS fine-grain
-         * runs of FMB_CHUNK sub-tiles per CTA at the end of the launch, so that the CTAs finish together.
-         * Smaller batches (64 streams on 444 CTAs) keep the static split into equal runs: a whole stream
-         * would be several CTAs' share.  FMB_CHUNK / FMB_TAIL_PCT (percent of the streams handed out in
-         * fine-grain runs) override the policy, for tuning and tests; FMB_CHUNK=0 forces the static split. */
-        const int spb = h->n_dem / FMB_NSUB;
-        const long long units = (long long) cfg->n_streams * spb;
-        const char *ec = getenv("FMB_CHUNK"), *et = getenv("FMB_TAIL_PCT");
-        const int chunk = ec ? atoi(ec) : FMB_DEFAULT_CHUNK;
-        const bool forced = ec || et;
-        for (fmb_handle::Plan *pl : {&h->plan, &h->plan_ws}) {
-            if (!(pl->ctas_per_sm > 0 && chunk > 0 && chunk <= spb && spb % chunk == 0 &&
-                  (forced || units >= 2LL * spb * pl->grid)))
-                continue;
-            int tail_streams;
-            if (et) {
-                int tail = atoi(et);
-                tail = tail < 0 ? 0 : tail > 100 ? 100 : tail;
-                tail_streams = cfg->n_streams - (int) ((long long) cfg->n_streams * (100 - tail) / 100);
-            } else if (h->pdl) {
-                /* overlapping launches: the CTAs of the next launch take over the slots this launch's ragged end
-                 * frees, so nothing has to finish together -- every stream is handed out whole (no lead-ins to
-                 * recompute).  1024 streams: 0.3475 -> 0.3337 ms per step (profiles/r02g_pdl_tail_sweep.txt) */
-                tail_streams = 0;
-            } else {
-                tail_streams = (FMB_DEFAULT_TAIL_RUNS * chunk * pl->grid + spb - 1) / spb;
-                if (tail_streams > cfg->n_streams) tail_streams = cfg->n_streams;
-            }
-            pl->chunk = chunk;
-            pl->n_whole = cfg->n_streams - tail_streams;
-        }
     }
     {
         /* the de-emphasis pass runs beside the NEXT step's demod kernel: give it the highest priority
@@ -639,6 +730,8 @@ int fmb_destroy(fmb_handle *h)
         if (h->ev_deemph[i]) cudaEventDestroy(h->ev_deemph[i]);
     }
     if (h->d_de_state) cudaFree(h->d_de_state);
+    if (h->d_seg_state) cudaFree(h->d_seg_state);
+    if (h->d_seg_count) cudaFree(h->d_seg_count);
     if (h->d_fallbacks) cudaFree(h->d_fallbacks);
     if (h->d_tickets) cudaFree(h->d_tickets);
     if (h->d_done) cudaFree(h->d_done);
@@ -680,6 +773,7 @@ int fmb_reset(fmb_handle *h)
     const size_t st_bytes = sizeof(fmb_stream_state) * (size_t) h->cfg.n_streams;
     for (int i = 0; i < 2; ++i) CU(cudaMemset(h->d_state[i], 0, st_bytes));
     CU(cudaMemset(h->d_de_state, 0, sizeof(float) * 2 * (size_t) h->cfg.n_streams));
+    if (h->d_seg_count) CU(cudaMemset(h->d_seg_count, 0, sizeof(unsigned int) * (size_t) h->cfg.n_streams));
     /* The ticket counters run on.  The stream hand-over counters stand at 2*seq after a clean run (what the next
      * launch waits for); they are set to that explicitly so that reset also recovers a handle whose flag wait timed
      * out, and the error word is cleared. */
@@ -705,7 +799,22 @@ int fmb_reset(fmb_handle *h)
     return FMB_OK;
 }
 
-int fmb_next_out_count(const fmb_handle *h) { return h ? out_count_for(h, h->phase) : FMB_ERR_ARG; }
+int fmb_set_blocks_per_call(fmb_handle *h, int n)
+{
+    if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
+    if (n < 1 || n > h->max_blocks) return set_err(FMB_ERR_ARG, "blocks per call must be in [1, max_blocks_per_call]");
+    h->blocks = n;
+    return FMB_OK;
+}
+
+int fmb_next_out_count(const fmb_handle *h) { return h ? out_count_for(h, h->phase, h->blocks) : FMB_ERR_ARG; }
+
+int fmb_out_count_blocks(const fmb_handle *h, int n_blocks)
+{
+    if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
+    if (n_blocks < 0 || n_blocks > h->max_blocks) return set_err(FMB_ERR_ARG, "n_blocks must be in [0, max_blocks_per_call]");
+    return out_count_for(h, h->phase, n_blocks);
+}
 int fmb_max_out_count(const fmb_handle *h) { return h ? h->max_out : FMB_ERR_ARG; }
 
 int fmb_process_device(fmb_handle *h, const uint8_t *iq_dev, size_t iq_pitch, int16_t *pcm_dev, size_t pcm_pitch,
@@ -755,11 +864,19 @@ static int ensure_slots(fmb_handle *h)
 {
     if (h->slot[0].d_iq) return FMB_OK;
     const fmb_config &c = h->cfg;
-    h->d_iq_pitch = (size_t) c.block_bytes;
+    h->d_iq_pitch = (size_t) h->max_blocks * c.block_bytes;
     h->d_pcm_pitch = ((size_t) h->max_out + 7) & ~(size_t) 7;
     for (auto &s : h->slot) {
-        CU(cudaMalloc(&s.d_iq, h->d_iq_pitch * c.n_streams));
-        CU(cudaMalloc(&s.d_pcm, h->d_pcm_pitch * c.n_streams * sizeof(int16_t)));
+        int rc = dev_alloc((void **) &s.d_iq, h->d_iq_pitch * c.n_streams, "pipeline IQ slot");
+        if (rc == FMB_OK) rc = dev_alloc((void **) &s.d_pcm, h->d_pcm_pitch * c.n_streams * sizeof(int16_t), "pipeline PCM slot");
+        if (rc != FMB_OK) {
+            for (auto &t : h->slot) {
+                if (t.d_iq) cudaFree(t.d_iq);
+                if (t.d_pcm) cudaFree(t.d_pcm);
+                t.d_iq = nullptr; t.d_pcm = nullptr;
+            }
+            return rc;
+        }
         CU(cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&s.ev_iq_free, cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&s.ev_done, cudaEventDisableTiming));
@@ -772,18 +889,19 @@ int fmb_submit(fmb_handle *h, const uint8_t *iq_host, size_t iq_pitch, int16_t *
 {
     if (!h || !iq_host || !pcm_host) return set_err(FMB_ERR_ARG, "NULL argument");
     const fmb_config &c = h->cfg;
-    if (iq_pitch < (size_t) c.block_bytes) return set_err(FMB_ERR_ARG, "iq_pitch < block_bytes");
+    const size_t row = (size_t) h->blocks * c.block_bytes;
+    if (iq_pitch < row) return set_err(FMB_ERR_ARG, "iq_pitch < blocks per call x block_bytes");
     CU(cudaSetDevice(c.device));
     int rc = ensure_slots(h);
     if (rc != FMB_OK) return rc;
     const int t = h->next_ticket;
     Slot &s = h->slot[t % FMB_PIPE_DEPTH];
     if (s.busy) return set_err(FMB_ERR_STATE, "pipeline full: fmb_wait() the oldest ticket first");
-    const int n_out = out_count_for(h, h->phase);
+    const int n_out = out_count_for(h, h->phase, h->blocks);
     if ((size_t) n_out > pcm_pitch) return set_err(FMB_ERR_ARG, "pcm_pitch smaller than fmb_next_out_count()");
 
     /* H2D on its own stream; the slot's previous demod has been waited for by the host (busy == false) */
-    CU(cudaMemcpy2DAsync(s.d_iq, h->d_iq_pitch, iq_host, iq_pitch, (size_t) c.block_bytes, (size_t) c.n_streams,
+    CU(cudaMemcpy2DAsync(s.d_iq, h->d_iq_pitch, iq_host, iq_pitch, row, (size_t) c.n_streams,
                          cudaMemcpyHostToDevice, h->s_h2d));
     CU(cudaEventRecord(s.ev_h2d, h->s_h2d));
     CU(cudaStreamWaitEvent(h->s_main, s.ev_h2d, 0));
@@ -948,7 +1066,11 @@ int fmb_debug_enable(fmb_handle *h, int on)
 {
     if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
     CU(cudaSetDevice(h->cfg.device));
-    if (on && !h->d_dem) CU(cudaMalloc(&h->d_dem, sizeof(float) * (size_t) h->n_dem * h->cfg.n_streams));
+    if (on && !h->d_dem) {
+        const int rc = dev_alloc((void **) &h->d_dem, sizeof(float) * (size_t) h->max_blocks * h->n_dem * h->cfg.n_streams,
+                                 "debug tap");
+        if (rc != FMB_OK) return rc;
+    }
     h->debug = on ? 1 : 0;
     return FMB_OK;
 }
@@ -960,8 +1082,9 @@ int fmb_debug_read(fmb_handle *h, float *dem_host, size_t dem_pitch, float *lr_h
     CU(cudaSetDevice(h->cfg.device));
     CU(cudaDeviceSynchronize());
     if (dem_host) {
-        if (dem_pitch < (size_t) h->n_dem) return set_err(FMB_ERR_ARG, "dem_pitch too small");
-        CU(cudaMemcpy2D(dem_host, dem_pitch * 4, h->d_dem, (size_t) h->n_dem * 4, (size_t) h->n_dem * 4,
+        const size_t n_dem = (size_t) h->last_blocks * h->n_dem;   /* the last call's row */
+        if (dem_pitch < n_dem) return set_err(FMB_ERR_ARG, "dem_pitch too small");
+        CU(cudaMemcpy2D(dem_host, dem_pitch * 4, h->d_dem, (size_t) h->max_blocks * h->n_dem * 4, n_dem * 4,
                         (size_t) h->cfg.n_streams, cudaMemcpyDeviceToHost));
     }
     if (lr_host && h->last_n_out > 0) {

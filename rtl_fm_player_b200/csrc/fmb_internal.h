@@ -43,6 +43,8 @@ int fmb_design_tables(const fmb_config *cfg, fmb_tables *t);
 #define FMB_DEFAULT_CHUNK 2        /* sub-tiles per fine-grain run, 0 = static split (env FMB_CHUNK)   */
 #define FMB_DEFAULT_TAIL_RUNS 2    /* fine-grain runs per CTA at the end of a launch (env FMB_TAIL_PCT overrides) */
 #define FMB_WARM 256               /* recomputed lead-in of a segment that is not first  */
+#define FMB_DE_CHUNK 1024          /* values a de-emphasis warp walks per step (fmb_deemph_kernel)         */
+#define FMB_DE_MIN_SEG_CHUNKS 8    /* shortest time segment of a long row in the de-emphasis passes, in chunks */
 
 typedef struct fmb_kparams {
     const uint8_t *iq;             /* [stream][iq_pitch] bytes, this step's block        */
@@ -55,11 +57,13 @@ typedef struct fmb_kparams {
     long long dem_pitch;
     int n_streams;
     int grid;                      /* CTAs: the (stream, sub-tile) units are dealt out evenly */
-    int n_dem;                     /* demodulated samples per stream this step            */
+    int n_dem;                     /* demodulated samples per stream this step (the whole row of its blocks) */
     int slow, fast, phase0;        /* resampler: rate_out2, rate_out, prev_lpr_index      */
     int dec;                       /* fast/slow when integral, else 0                     */
     int dec_c0;                    /* tick at relative i  <=>  (i + dec_c0) % dec == dec-1 */
-    int quirk;                     /* patch d[1] with R of the tick at i=0 (SURVEY A.7)   */
+    int blk_dem;                   /* demodulated samples per reference block; at every block start of the row whose
+                                      phase puts a tick on its sample 0, patch sample 1 with R of that tick (in-place
+                                      quirk, SURVEY A.7).  0: not emulated                                          */
     /* Dynamic work assignment (chunk > 0): see "work assignment" in fmb_demod_kernel. */
     int chunk;                     /* units per fine-grain run; divides n_dem / FMB_NSUB  */
     int n_whole;                   /* streams handed out whole before the fine-grain runs */
@@ -98,6 +102,12 @@ typedef struct fmb_dparams {
     unsigned int *fallbacks;       /* device counter: chunks whose time-speculation failed and
                                       were redone sequentially (diagnostic; may be NULL)   */
     unsigned int *de_done;         /* [n_streams] += 1 when this pass is done with the stream's input row        */
+    /* Time segments of a long row (segs > 1: fmb_deemph_seg_kernel instead of fmb_deemph_kernel) */
+    int segs;                      /* segments per stream, 1 = one warp walks the whole row                       */
+    int seg_chunks;                /* 1024-value chunks per segment (the last one may have fewer)                 */
+    float *seg_state;              /* [stream][segs][4]: assumed start (l, r) and end (l, r) of each segment      */
+    unsigned int *seg_count;       /* [stream]: segments finished in this pass; the last one walks the junctions
+                                      and sets it back to 0                                                       */
 } fmb_dparams;
 
 /* Sets fmb_last_error() of the calling thread (host code outside fmb_api.cu reports through it). */
@@ -106,6 +116,8 @@ void fmb_set_last_error(const char *msg);
 /* Launchers (fmb_kernels.cu).  `stream` is a cudaStream_t.  Return cudaError_t as int. */
 int fmb_launch_demod(const fmb_config *cfg, const fmb_kparams *p, const fmb_tables *t, void *stream);
 int fmb_launch_deemph(const fmb_dparams *p, void *stream);
+/* resident warps per SM of the de-emphasis passes (sizes the time segments of long rows) */
+int fmb_deemph_occupancy(int *warps_per_sm);
 /* resident CTAs per SM of the kernel this configuration selects */
 int fmb_demod_occupancy(const fmb_config *cfg, int *ctas_per_sm);
 int fmb_demod_ws_occupancy(const fmb_config *cfg, int *ctas_per_sm);

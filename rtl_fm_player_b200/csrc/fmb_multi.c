@@ -201,6 +201,20 @@ fmb_handle *fmb_multi_handle(fmb_multi *m, int shard)
 }
 
 int fmb_multi_next_out_count(const fmb_multi *m) { return m ? fmb_next_out_count(m->sh[0].h) : FMB_ERR_ARG; }
+int fmb_multi_out_count_blocks(const fmb_multi *m, int n_blocks)
+{
+    return m ? fmb_out_count_blocks(m->sh[0].h, n_blocks) : fail_arg("NULL handle");
+}
+
+int fmb_multi_set_blocks_per_call(fmb_multi *m, int n)
+{
+    int i, rc;
+    if (!m) return fail_arg("NULL handle");
+    /* host bookkeeping only: every shard accepts the same n (they share the configuration) */
+    for (i = 0; i < m->n; ++i)
+        if ((rc = fmb_set_blocks_per_call(m->sh[i].h, n)) != FMB_OK) return rc;
+    return FMB_OK;
+}
 int fmb_multi_max_out_count(const fmb_multi *m) { return m ? m->max_out : FMB_ERR_ARG; }
 
 int fmb_multi_reset(fmb_multi *m)

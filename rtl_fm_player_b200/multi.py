@@ -62,6 +62,7 @@ class FmMulti:
         dv = (C.c_int * len(devices))(*devices)
         L.check(self._lib.fmb_multi_create(C.byref(cc), dv, len(devices), C.byref(self._m)), "fmb_multi_create")
         self.max_out = self._lib.fmb_multi_max_out_count(self._m)
+        self._blocks = cfg.max_blocks
         self.shards = []
         for g in range(self._lib.fmb_multi_shards(self._m)):
             first, count, dev = C.c_int(), C.c_int(), C.c_int()
@@ -89,6 +90,13 @@ class FmMulti:
     def next_out_count(self) -> int:
         return L.check(self._lib.fmb_multi_next_out_count(self._m), "fmb_multi_next_out_count")
 
+    def set_blocks_per_call(self, n: int) -> None:
+        L.check(self._lib.fmb_multi_set_blocks_per_call(self._m, n), "fmb_multi_set_blocks_per_call")
+        self._blocks = n
+
+    def out_count_blocks(self, n_blocks: int) -> int:
+        return L.check(self._lib.fmb_multi_out_count_blocks(self._m, n_blocks), "fmb_multi_out_count_blocks")
+
     def reset(self) -> None:
         L.check(self._lib.fmb_multi_reset(self._m), "fmb_multi_reset")
 
@@ -104,8 +112,13 @@ class FmMulti:
         L.check(self._lib.fmb_multi_wait(self._m, ticket, None), "fmb_multi_wait")
 
     def process(self, iq: np.ndarray, pcm: np.ndarray | None = None) -> np.ndarray:
-        """iq: uint8 [n_streams, block_bytes] (ideally pinned_array) -> int16 [n_streams, n_out]."""
-        S, B = self.cfg.n_streams, self.cfg.block_bytes
+        """iq: uint8 [n_streams, m * block_bytes], 1 <= m <= max_blocks_per_call (ideally pinned_array)
+        -> int16 [n_streams, n_out]."""
+        S = self.cfg.n_streams
+        m = iq.shape[1] // self.cfg.block_bytes
+        if m != self._blocks:
+            self.set_blocks_per_call(m)
+        B = m * self.cfg.block_bytes
         assert iq.dtype == np.uint8 and iq.shape == (S, B) and iq.flags.c_contiguous and iq.ctypes.data % 16 == 0
         n = self.next_out_count()
         pitch = max(8, (n + 7) & ~7)
@@ -120,13 +133,16 @@ class FmMulti:
 
     def run(self, iq: np.ndarray) -> np.ndarray:
         """Whole captures uint8 [n_streams, n_bytes]; full blocks only (demod_thread_fn :863-868)."""
-        S, B = self.cfg.n_streams, self.cfg.block_bytes
-        stage = pinned_array((S, B), np.uint8)
+        S, B, k = self.cfg.n_streams, self.cfg.block_bytes, self.cfg.max_blocks
+        n_blocks = iq.shape[1] // B
+        stage = pinned_array((S, k * B), np.uint8)
         outs = []
         try:
-            for b in range(iq.shape[1] // B):
-                stage[...] = iq[:, b * B:(b + 1) * B]
-                outs.append(self.process(stage).copy())
+            for b in range(0, n_blocks, k):
+                m = min(k, n_blocks - b)
+                st = stage[:, :m * B] if m == k else np.ascontiguousarray(stage[:, :m * B])
+                st[...] = iq[:, b * B:(b + m) * B]
+                outs.append(self.process(st).copy())
         finally:
             free_pinned(stage)
         return np.concatenate(outs, axis=1) if outs else np.empty((S, 0), dtype=np.int16)
