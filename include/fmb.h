@@ -100,8 +100,22 @@ int fmb_preset_mono_192k(fmb_config *cfg);
 int fmb_create(const fmb_config *cfg, fmb_handle **out);
 int fmb_destroy(fmb_handle *h);
 
-/* demod_state.volume may change while the player runs; takes effect from the next process call. */
+/* demod_state.volume may change while the player runs; takes effect from the next process call.  Sets the volume of
+ * every stream, also of those given their own with fmb_set_stream_output. */
 int fmb_set_volume(fmb_handle *h, float volume);
+
+/* Output settings of streams [first, first+count); NULL array = keep that setting.  deemph in seconds (0 = off);
+ * deemph_lambda > 0 overrides the pole as fmb_config.deemph_lambda does.  Takes effect from the next
+ * process/submit call; submits in flight keep the settings they were submitted with.
+ * Every stream starts with the handle's own (cfg.volume, cfg.deemph, cfg.deemph_lambda), and each keeps the reference's
+ * per-player meaning (demod_state.volume / deemph / deemph_lambda): stream s of a mixed batch produces bit for bit what a
+ * one-stream handle created with s's settings produces.  fmb_reset keeps them.  FMB_ERR_ARG, with nothing applied, for a
+ * range outside the handle, a non-finite volume, a negative or non-finite deemph, or a deemph_lambda outside [0, 1). */
+int fmb_set_stream_output(fmb_handle *h, int first, int count, const float *volume, const double *deemph,
+                          const float *deemph_lambda);
+/* The settings of streams [first, first+count): volume, the de-emphasis pole in effect (0 when off) and whether
+ * de-emphasis is on; NULL array = not wanted. */
+int fmb_get_stream_output(const fmb_handle *h, int first, int count, float *volume, float *lambda, int *deemph_on);
 
 /* Back to stream start: every stage's history zero in its own float domain,
  * as after demod_init + init_lp_real_f32 (:1156, :413). */
@@ -167,6 +181,10 @@ void *fmb_internal_stream(fmb_handle *h);
 /* Which demodulation kernel the NEXT process call launches ("fmb_demod_kernel", or "fmb_mono_ws_kernel": the
  * warp-specialised kernel of the mono decoder); for profiles and the benchmark. */
 const char *fmb_demod_kernel_name(const fmb_handle *h);
+/* Which de-emphasis kernel the NEXT process call launches: "fmb_deemph_kernel", or "fmb_deemph_seg_kernel" when the
+ * call's rows are split into time segments; with the suffix "_per_stream" when some stream's output settings differ
+ * from the handle's own (fmb_set_stream_output), so that the pass reads them from a per-stream table. */
+const char *fmb_deemph_kernel_name(const fmb_handle *h);
 /* Blocks until the handle's device has finished everything enqueued so far. */
 int fmb_sync(fmb_handle *h);
 

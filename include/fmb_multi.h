@@ -50,6 +50,11 @@ int fmb_multi_max_out_count(const fmb_multi *m);
 int fmb_multi_set_blocks_per_call(fmb_multi *m, int n);
 int fmb_multi_out_count_blocks(const fmb_multi *m, int n_blocks);
 int fmb_multi_reset(fmb_multi *m);
+/* fmb_set_stream_output / fmb_get_stream_output over GLOBAL stream indices [first, first+count): the range is split over
+ * the shards it covers (fmb_multi_shard_range).  The arguments are checked for the whole range before any shard changes. */
+int fmb_multi_set_stream_output(fmb_multi *m, int first, int count, const float *volume, const double *deemph,
+                                const float *deemph_lambda);
+int fmb_multi_get_stream_output(const fmb_multi *m, int first, int count, float *volume, float *lambda, int *deemph_on);
 
 /* As fmb_submit / fmb_wait / fmb_process, for the whole batch: iq_host[s*iq_pitch ...] is stream s's
  * block, pcm_host[s*pcm_pitch ...] receives its PCM (pitch in int16 units).  Up to FMB_PIPE_DEPTH

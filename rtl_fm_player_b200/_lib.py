@@ -89,6 +89,11 @@ SIGNATURES = {
     "fmb_internal_stream": (C.c_void_p, [C.c_void_p]),
     "fmb_sync": (C.c_int, [C.c_void_p]),
     "fmb_demod_kernel_name": (C.c_char_p, [C.c_void_p]),
+    "fmb_deemph_kernel_name": (C.c_char_p, [C.c_void_p]),
+    "fmb_set_stream_output": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_double),
+                                        C.POINTER(C.c_float)]),
+    "fmb_get_stream_output": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float),
+                                        C.POINTER(C.c_int)]),
     # include/fmb_multi.h: the C multi-GPU host (one worker thread per device)
     "fmb_multi_create": (C.c_int, [C.POINTER(FmbConfig), C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_void_p)]),
     "fmb_multi_destroy": (C.c_int, [C.c_void_p]),
@@ -100,6 +105,10 @@ SIGNATURES = {
     "fmb_multi_out_count_blocks": (C.c_int, [C.c_void_p, C.c_int]),
     "fmb_multi_max_out_count": (C.c_int, [C.c_void_p]),
     "fmb_multi_reset": (C.c_int, [C.c_void_p]),
+    "fmb_multi_set_stream_output": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                              C.POINTER(C.c_double), C.POINTER(C.c_float)]),
+    "fmb_multi_get_stream_output": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                              C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "fmb_multi_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),
     "fmb_multi_wait": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int)]),
     "fmb_multi_process": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),
@@ -136,6 +145,28 @@ def lib() -> C.CDLL:
             fn.argtypes = args
         _lib = L
     return _lib
+
+
+def stream_output_args(n_streams: int, first: int, volume, deemph, deemph_lambda):
+    """(count, volume, deemph, deemph_lambda) for fmb[_multi]_set_stream_output: each setting None (keep), a scalar
+    broadcast over the range or an array of its length.  The range is [first, first + len) of the arrays given, or
+    [first, n_streams) when every setting is a scalar."""
+    import numpy as np
+    given = [(v, t) for v, t in ((volume, np.float32), (deemph, np.float64), (deemph_lambda, np.float32))]
+    lens = {np.size(v) for v, _ in given if v is not None and np.ndim(v) > 0}
+    if len(lens) > 1:
+        raise ValueError(f"per-stream settings of different lengths {sorted(lens)}")
+    count = lens.pop() if lens else n_streams - first
+    out = []
+    for v, t in given:
+        if v is None:
+            out.append((None, None))
+        else:
+            a = np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=t), (count,)))
+            ct = C.c_double if t is np.float64 else C.c_float
+            out.append((a, a.ctypes.data_as(C.POINTER(ct))))
+    # the arrays are returned with their pointers so that they outlive the call
+    return count, out
 
 
 def check(rc: int, where: str) -> int:

@@ -113,8 +113,30 @@ class FmBatch:
     def kernel_name(self) -> str:
         return self._lib.fmb_demod_kernel_name(self._h).decode()
 
+    def deemph_kernel_name(self) -> str:
+        """The de-emphasis kernel the next call launches (fmb_deemph_kernel_name)."""
+        return self._lib.fmb_deemph_kernel_name(self._h).decode()
+
     def set_volume(self, volume: float) -> None:
+        """Volume of every stream (fmb_set_volume)."""
         L.check(self._lib.fmb_set_volume(self._h, volume), "fmb_set_volume")
+
+    def set_stream_output(self, volume=None, deemph=None, deemph_lambda=None, first: int = 0) -> None:
+        """Output settings of streams [first, first + n) from the next call on (fmb_set_stream_output): volume,
+        de-emphasis time constant in seconds (0 = off) and pole override (> 0).  None keeps a setting; a scalar is
+        broadcast over the range, an array gives one value per stream and n is its length (with scalars only, the
+        range runs to the last stream)."""
+        count, args = L.stream_output_args(self.cfg.n_streams, first, volume, deemph, deemph_lambda)
+        L.check(self._lib.fmb_set_stream_output(self._h, first, count, *(p for _, p in args)), "fmb_set_stream_output")
+
+    def stream_output(self, first: int = 0, count: int | None = None) -> dict:
+        """{"volume", "lambda", "deemph_on"} of streams [first, first + count) (fmb_get_stream_output)."""
+        count = self.cfg.n_streams - first if count is None else count
+        vol, lam, on = (np.empty(count, np.float32), np.empty(count, np.float32), np.empty(count, np.int32))
+        L.check(self._lib.fmb_get_stream_output(self._h, first, count, vol.ctypes.data_as(C.POINTER(C.c_float)),
+                                                lam.ctypes.data_as(C.POINTER(C.c_float)),
+                                                on.ctypes.data_as(C.POINTER(C.c_int))), "fmb_get_stream_output")
+        return {"volume": vol, "lambda": lam, "deemph_on": on.astype(bool)}
 
     def reset(self) -> None:
         L.check(self._lib.fmb_reset(self._h), "fmb_reset")

@@ -31,6 +31,16 @@ static float windowed_band(float lo, float hi, float pos, float win)
     return v * win;
 }
 
+/* de-emphasis pole at the OUTPUT rate (:1577; output.rate follows -r, :1416-1419) */
+float fmb_deemph_pole(const fmb_config *cfg, double deemph, float deemph_lambda)
+{
+    const int fast = cfg->rate_out > 0 ? cfg->rate_out : cfg->rate_in;          /* output.rate = demod.rate_out, :1512-1514 */
+    const int out_rate = cfg->rate_out2 > 0 ? cfg->rate_out2 : fast;
+    if (deemph == 0.0) return 0.0f;
+    if (deemph_lambda > 0.0f) return deemph_lambda;
+    return (float) exp(-1.0 / ((double) out_rate * deemph));
+}
+
 int fmb_design_tables(const fmb_config *cfg, fmb_tables *t)
 {
     const float rate = (float) cfg->rate_in;
@@ -68,13 +78,7 @@ int fmb_design_tables(const fmb_config *cfg, fmb_tables *t)
         }
     }
 
-    /* de-emphasis pole at the OUTPUT rate (:1577; output.rate follows -r, :1416-1419) */
-    {
-        const int fast = cfg->rate_out > 0 ? cfg->rate_out : cfg->rate_in;          /* output.rate = demod.rate_out, :1512-1514 */
-        const int out_rate = cfg->rate_out2 > 0 ? cfg->rate_out2 : fast;
-        t->lambda = cfg->deemph != 0.0 ? (float) exp(-1.0 / ((double) out_rate * cfg->deemph)) : 0.0f;
-        if (cfg->deemph != 0.0 && cfg->deemph_lambda > 0.0f) t->lambda = cfg->deemph_lambda;
-    }
+    t->lambda = fmb_deemph_pole(cfg, cfg->deemph, cfg->deemph_lambda);
     t->pcm_scale = cfg->volume * 32768.0f; /* :717 */
     t->one = 1.0f;
     return FMB_OK;

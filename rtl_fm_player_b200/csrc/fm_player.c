@@ -14,6 +14,7 @@
  * Flags follow the reference's where they exist (-X -Y -s -r -E offset, :1389-1508).
  */
 #define _POSIX_C_SOURCE 200809L
+#include <math.h>
 #include <pthread.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -99,9 +100,12 @@ static void usage(void)
     fprintf(stderr,
             "fmb_player -- batched offline FM demodulator (B200), one rtl_sdr-format uint8 IQ capture per channel\n"
             "usage: fmb_player [-X | -Y] [-s rate_in] [-r rate_out2] [-E offset] [-m lpr_mode] [-z lpr_size]\n"
-            "                  [-v volume] [-w] [-o out_dir] [-d cuda_devices] [-P exact|fma] [-R speed] [-K blocks]\n"
-            "                  capture.u8 ...\n"
+            "                  [-v volume] [-e deemph_us] [-w] [-o out_dir] [-d cuda_devices] [-P exact|fma] [-R speed]\n"
+            "                  [-K blocks] (capture.u8 ... | -M manifest)\n"
             "  -X  stereo preset 192k/48k, 90 taps   -Y  mono preset 192k/48k, 128 taps   (as rtl_fm_player)\n"
+            "  -e  de-emphasis time constant in microseconds, 0 = off (default 50); holds wherever -X / -Y stand\n"
+            "  -M  channels from a file instead of the command line, one per line: `path [volume] [deemph_us]`;\n"
+            "      a missing field takes -v / -e.  Each channel's output is what running it alone with those settings gives\n"
             "  -w  write <name>.wav with the reference's header and 32768-byte cluster rule (default: raw <name>.pcm)\n"
             "  -d  CUDA devices to shard the channels over, e.g. 0-7 or 0,2,4 (default 0); at least one channel per device\n"
             "  -R  pace the captures at `speed` x real time (default: as fast as the GPU takes them)\n"
@@ -115,6 +119,24 @@ static const char *base_name(const char *path)
     return s ? s + 1 : path;
 }
 
+/* One manifest line: "path [volume] [deemph_us]" (blank lines and lines starting with '#' are skipped: returns 0).
+ * Returns 1 for a channel, -1 for a malformed line. */
+static int parse_manifest_line(char *line, char **path, float *volume, double *deemph)
+{
+    char *f[4], *save = NULL, *t, *end;
+    int n = 0;
+    for (t = strtok_r(line, " \t\r\n", &save); t; t = strtok_r(NULL, " \t\r\n", &save)) {
+        if (n == 4) return -1;
+        f[n++] = t;
+    }
+    if (n == 0 || f[0][0] == '#') return 0;
+    if (n > 3) return -1;
+    *path = f[0];
+    if (n > 1) { *volume = strtof(f[1], &end); if (end == f[1] || *end || !isfinite(*volume)) return -1; }
+    if (n > 2) { *deemph = strtod(f[2], &end) / 1e6; if (end == f[2] || *end || !(isfinite(*deemph) && *deemph >= 0.0)) return -1; }
+    return 1;
+}
+
 int main(int argc, char **argv)
 {
     struct player P;
@@ -126,6 +148,12 @@ int main(int argc, char **argv)
     int *n_outs;
     int devices[64], n_devices = 1;
     fmb_multi *h = NULL;
+    const char *manifest = NULL;
+    double deemph_arg = -1.0;   /* -e in seconds, applied after all flags so that a preset given later does not undo it */
+    char **paths = NULL;        /* per channel: capture file */
+    float *volumes = NULL;      /* per channel: -v or the manifest's */
+    double *deemphs = NULL;     /* per channel: -e or the manifest's, in seconds */
+    int have_manifest_settings = 0;
 
     memset(&P, 0, sizeof P);
     P.K = 1;
@@ -141,6 +169,16 @@ int main(int argc, char **argv)
         else if (!strcmp(a, "-m") && i + 1 < argc) P.cfg.mode = atoi(argv[++i]);
         else if (!strcmp(a, "-z") && i + 1 < argc) P.cfg.size = atoi(argv[++i]);
         else if (!strcmp(a, "-v") && i + 1 < argc) P.cfg.volume = (float) atof(argv[++i]);
+        else if (!strcmp(a, "-e") && i + 1 < argc) {
+            char *end;
+            const char *v = argv[++i];
+            deemph_arg = strtod(v, &end) / 1e6;             /* 50 -> 0.000050 exactly as demod_init's constant */
+            if (end == v || *end || !(isfinite(deemph_arg) && deemph_arg >= 0.0)) {
+                fprintf(stderr, "-e: need a finite number of microseconds >= 0\n");
+                return 2;
+            }
+        }
+        else if (!strcmp(a, "-M") && i + 1 < argc) manifest = argv[++i];
         else if (!strcmp(a, "-d") && i + 1 < argc) {
             n_devices = fmb_parse_device_list(argv[++i], devices, 64);
             if (n_devices < 1) { fprintf(stderr, "-d: %s\n", fmb_last_error()); return 2; }
@@ -154,9 +192,45 @@ int main(int argc, char **argv)
         else if (a[0] == '-' && a[1]) { usage(); return 2; }
         else { first_file = i; break; }
     }
-    if (first_file < 0) { usage(); return 2; }
     if (P.K < 1) { fprintf(stderr, "-K: need at least one block per step\n"); return 2; }
-    P.n = argc - first_file;
+    if (deemph_arg >= 0.0) P.cfg.deemph = deemph_arg;
+    if (manifest) {
+        FILE *mf;
+        char line[4096];
+        int ln = 0, cap = 0;
+        if (first_file >= 0) { fprintf(stderr, "-M: give the channels either in the manifest or on the command line\n"); return 2; }
+        mf = fopen(manifest, "r");
+        if (!mf) { perror(manifest); return 2; }
+        while (fgets(line, sizeof line, mf)) {
+            char *path;
+            float vol = P.cfg.volume;
+            double de = P.cfg.deemph;
+            int r;
+            ++ln;
+            r = parse_manifest_line(line, &path, &vol, &de);
+            if (r < 0) { fprintf(stderr, "%s:%d: malformed line (want `path [volume] [deemph_us]`)\n", manifest, ln); fclose(mf); return 2; }
+            if (r == 0) continue;
+            if (P.n == cap) {
+                cap = cap ? 2 * cap : 16;
+                paths = realloc(paths, (size_t) cap * sizeof *paths);
+                volumes = realloc(volumes, (size_t) cap * sizeof *volumes);
+                deemphs = realloc(deemphs, (size_t) cap * sizeof *deemphs);
+                if (!paths || !volumes || !deemphs) return 1;
+            }
+            paths[P.n] = strdup(path);
+            if (!paths[P.n]) return 1;
+            volumes[P.n] = vol;
+            deemphs[P.n] = de;
+            if (vol != P.cfg.volume || de != P.cfg.deemph) have_manifest_settings = 1;
+            P.n++;
+        }
+        fclose(mf);
+        if (P.n == 0) { fprintf(stderr, "%s: no channels\n", manifest); return 2; }
+    } else {
+        if (first_file < 0) { usage(); return 2; }
+        P.n = argc - first_file;
+        paths = argv + first_file;
+    }
     P.cfg.n_streams = P.n;
     P.cfg.max_blocks_per_call = P.K;
     P.row = (size_t) P.K * (size_t) P.cfg.block_bytes;
@@ -170,6 +244,10 @@ int main(int argc, char **argv)
     if (n_devices == 1) fmb_bind_thread_to_device_node(devices[0]); /* best effort: node-local pinned buffers */
     rc = fmb_multi_create(&P.cfg, devices, n_devices, &h);
     if (rc != FMB_OK) { fprintf(stderr, "fmb_multi_create: %s\n", fmb_last_error()); return 1; }
+    if (have_manifest_settings) {
+        rc = fmb_multi_set_stream_output(h, 0, P.n, volumes, deemphs, NULL);
+        if (rc != FMB_OK) { fprintf(stderr, "%s: %s\n", manifest, fmb_last_error()); return 2; }
+    }
     P.pcm_pitch = ((size_t) fmb_multi_max_out_count(h) + 7) & ~(size_t) 7;
     for (i = 0; i < NBUF; ++i) {
         if (fmb_host_alloc((void **) &P.iq[i], (size_t) P.n * P.row) != FMB_OK ||
@@ -183,7 +261,7 @@ int main(int argc, char **argv)
     for (i = 0; i < P.n; ++i) {
         struct chan *c = &P.ch[i];
         char path[4096];
-        const char *in = argv[first_file + i];
+        const char *in = paths[i];
         c->p = &P; c->index = i;
         if (filesrc_open(&c->src, in) != 0) { perror(in); return 1; }
         filesrc_set_sample_rate(c->src, (uint32_t) (8 * P.cfg.rate_in)); /* capture_rate, :1053 */
@@ -267,5 +345,11 @@ int main(int argc, char **argv)
     fmb_multi_destroy(h);
     free(P.ch);
     free(n_outs);
+    if (manifest) {
+        for (i = 0; i < P.n; ++i) free(paths[i]);
+        free(paths);
+    }
+    free(volumes);
+    free(deemphs);
     return 0;
 }

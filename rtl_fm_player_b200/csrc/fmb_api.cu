@@ -14,6 +14,7 @@
 
 #include <atomic>
 #include <cctype>
+#include <cmath>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
@@ -28,6 +29,9 @@ static_assert(offsetof(fmb_stream_state, raw_tail) % 16 == 0 && sizeof(fmb_strea
 namespace {
 
 constexpr int kLrBufs = FMB_LR_BUFS;
+/* pinned snapshots of the per-stream output table: a change between calls is uploaded from the next free one, so the
+ * host rarely waits for an upload FMB_PIPE_DEPTH changes back before it may overwrite the snapshot */
+constexpr int kOutStage = FMB_PIPE_DEPTH;
 
 thread_local char g_err[512] = "";
 std::atomic<long> g_launches{0};
@@ -129,6 +133,18 @@ struct fmb_handle {
     int pcount[2] = {0, 0};
     double pms[2] = {0, 0};
     int plaunch[2] = {0, 0};
+    /* per-stream output settings (fmb_set_stream_output): as given, and as the de-emphasis passes read them */
+    float *out_volume = nullptr;      /* [n_streams] */
+    double *out_deemph = nullptr;     /* [n_streams] seconds, 0 = off */
+    float *out_lambda_set = nullptr;  /* [n_streams] deemph_lambda override, 0 = none */
+    fmb_stream_out *out_tab = nullptr;/* [n_streams] */
+    int out_differ = 0;               /* streams whose settings differ from the handle's own: 0 = the uniform launch */
+    unsigned long long out_version = 0, out_uploaded = 0; /* changes of out_tab; the one d_out_tab holds */
+    fmb_stream_out *d_out_tab = nullptr;                  /* device copy, read by the per-stream passes */
+    fmb_stream_out *h_out_stage[kOutStage] = {};          /* pinned snapshots, one per upload in flight */
+    cudaEvent_t ev_out_stage[kOutStage] = {};             /* that snapshot's upload has been executed */
+    bool out_stage_pending[kOutStage] = {};
+    int out_stage_next = 0;
 };
 
 namespace {
@@ -350,6 +366,87 @@ void deemph_segments(const fmb_handle *h, int n_blocks, int n_out, int *segs, in
     *segs = (int) ((n_chunk + per - 1) / per);
 }
 
+/* The table entry of stream s from its settings as given */
+fmb_stream_out stream_out_entry(const fmb_handle *h, int s)
+{
+    fmb_stream_out o;
+    o.do_deemph = h->out_deemph[s] != 0.0;
+    o.lambda = fmb_deemph_pole(&h->cfg, h->out_deemph[s], h->out_lambda_set[s]);
+    o.pcm_scale = h->out_volume[s] * 32768.0f;  /* :717, in float like the reference */
+    o.pad = 0;
+    return o;
+}
+
+/* Does stream s apply something else than the handle's own settings (those the uniform launch passes)? */
+bool stream_out_differs(const fmb_handle *h, int s)
+{
+    const fmb_stream_out &o = h->out_tab[s];
+    const bool on = h->cfg.deemph != 0.0;
+    if ((o.do_deemph != 0) != on) return true;
+    if (on && memcmp(&o.lambda, &h->tab.lambda, sizeof(float)) != 0) return true;
+    return memcmp(&o.pcm_scale, &h->tab.pcm_scale, sizeof(float)) != 0;
+}
+
+/* after a change of settings: recount the differing streams; the next per-stream pass uploads the table again */
+void stream_out_changed(fmb_handle *h)
+{
+    int n = 0;
+    for (int s = 0; s < h->cfg.n_streams; ++s) n += stream_out_differs(h, s);
+    h->out_differ = n;
+    h->out_version++;
+}
+
+/* The per-stream table the de-emphasis pass of this step reads, uploaded on `st` (the pass's stream, so the upload is
+ * ordered after every earlier pass and before this one) when it changed since the last upload.  NULL: every stream
+ * carries the handle's own settings, and the pass is the uniform launch.  Nothing is enqueued on failure. */
+int stream_out_for_step(fmb_handle *h, cudaStream_t st, const fmb_stream_out **out)
+{
+    *out = nullptr;
+    if (h->out_differ == 0) return FMB_OK;
+    const size_t bytes = sizeof(fmb_stream_out) * (size_t) h->cfg.n_streams;
+    if (!h->d_out_tab) {
+        /* all or nothing: a failure frees what this call allocated, so the next call starts over */
+        fmb_stream_out *d = nullptr;
+        fmb_stream_out *stage[kOutStage] = {};
+        cudaEvent_t ev[kOutStage] = {};
+        int rc = dev_alloc((void **) &d, bytes, "per-stream output table");
+        for (int i = 0; rc == FMB_OK && i < kOutStage; ++i) {
+            if (cudaHostAlloc((void **) &stage[i], bytes, cudaHostAllocDefault) != cudaSuccess ||
+                cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming) != cudaSuccess) {
+                cudaGetLastError();
+                rc = set_err(FMB_ERR_NOMEM, "per-stream output table staging");
+            }
+        }
+        if (rc != FMB_OK) {
+            if (d) cudaFree(d);
+            for (int i = 0; i < kOutStage; ++i) {
+                if (stage[i]) cudaFreeHost(stage[i]);
+                if (ev[i]) cudaEventDestroy(ev[i]);
+            }
+            return rc;
+        }
+        h->d_out_tab = d;
+        for (int i = 0; i < kOutStage; ++i) { h->h_out_stage[i] = stage[i]; h->ev_out_stage[i] = ev[i]; h->out_stage_pending[i] = false; }
+    }
+    if (h->out_uploaded != h->out_version) {
+        const int i = h->out_stage_next;
+        if (h->out_stage_pending[i]) CU(cudaEventSynchronize(h->ev_out_stage[i]));
+        h->out_stage_pending[i] = false;
+        memcpy(h->h_out_stage[i], h->out_tab, bytes);
+        CU(cudaMemcpyAsync(h->d_out_tab, h->h_out_stage[i], bytes, cudaMemcpyHostToDevice, st));
+        const cudaError_t e = cudaEventRecord(h->ev_out_stage[i], st);
+        if (e != cudaSuccess) {
+            cudaStreamSynchronize(st);   /* the staging buffer may be rewritten only once its upload has run */
+            return set_err(FMB_ERR_CUDA, "cudaEventRecord (per-stream output table upload)", e);
+        }
+        h->out_stage_pending[i] = true;
+        h->out_stage_next = (i + 1) % kOutStage;
+        h->out_uploaded = h->out_version;
+    }
+    *out = h->d_out_tab;
+    return FMB_OK;
+}
+
 /* Enqueue one step of h->blocks blocks: demod kernel on `sm`, de-emphasis kernel(s) on the aux
  * stream.  d_iq/d_pcm are device pointers. */
 int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d_pcm, size_t pcm_pitch,
@@ -381,6 +478,12 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
      * time-out at 8 mono streams x 16 blocks).  Such a pass is waited for here, and this launch does not overlap. */
     const bool wait_deemph = h->deemph_pending[b] && (!h->pdl || h->deemph_segmented[b]);
     if (wait_deemph) CU(cudaStreamWaitEvent(sm, h->ev_deemph[b], 0));
+    /* the per-stream output settings as they stand now: this step's pass reads this snapshot, whatever changes later */
+    const fmb_stream_out *out_tab = nullptr;
+    {
+        const int rc = stream_out_for_step(h, h->s_aux, &out_tab);
+        if (rc != FMB_OK) return rc;
+    }
 
     fmb_kparams kp;
     memset(&kp, 0, sizeof kp);
@@ -464,6 +567,7 @@ int enqueue_step(fmb_handle *h, const uint8_t *d_iq, size_t iq_pitch, int16_t *d
     deemph_segments(h, nb, n_out, &dp.segs, &dp.seg_chunks);
     dp.seg_state = h->d_seg_state;
     dp.seg_count = h->d_seg_count;
+    dp.out = out_tab;
     if (prof) CUP(cudaEventRecord(h->pev[1][0][h->pcount[1]], h->s_aux));
 #ifdef FMB_TUNE_SKIP_DEEMPH   /* tools/build_variant.sh only: timing experiment, PCM is not produced */
     e = cudaSuccess;
@@ -637,6 +741,23 @@ int fmb_create(const fmb_config *cfg, fmb_handle **out)
         h->env_chunk = ec ? (atoi(ec) > 0 ? atoi(ec) : 0) : -1;
         h->env_tail = et ? (atoi(et) > 0 ? atoi(et) : 0) : -1;
     }
+    {
+        const size_t n = (size_t) cfg->n_streams;
+        h->out_volume = (float *) malloc(sizeof(float) * n);
+        h->out_deemph = (double *) malloc(sizeof(double) * n);
+        h->out_lambda_set = (float *) malloc(sizeof(float) * n);
+        h->out_tab = (fmb_stream_out *) malloc(sizeof(fmb_stream_out) * n);
+        if (!h->out_volume || !h->out_deemph || !h->out_lambda_set || !h->out_tab) {
+            fmb_destroy(h);
+            return set_err(FMB_ERR_NOMEM, "per-stream output settings");
+        }
+        for (size_t s = 0; s < n; ++s) {
+            h->out_volume[s] = cfg->volume;
+            h->out_deemph[s] = cfg->deemph;
+            h->out_lambda_set[s] = cfg->deemph_lambda;
+            h->out_tab[s] = stream_out_entry(h, (int) s);
+        }
+    }
     h->phase = 0;
     h->blocks_done = 0;
     /* upper bound of outputs per step (at the most blocks per call) */
@@ -753,6 +874,15 @@ int fmb_destroy(fmb_handle *h)
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     for (int k = 0; k < 2; ++k)
         for (int e = 0; e < 2; ++e) destroy_events(h->pev[k][e], kProfMax);
+    if (h->d_out_tab) cudaFree(h->d_out_tab);
+    for (int i = 0; i < kOutStage; ++i) {
+        if (h->h_out_stage[i]) cudaFreeHost(h->h_out_stage[i]);
+        if (h->ev_out_stage[i]) cudaEventDestroy(h->ev_out_stage[i]);
+    }
+    free(h->out_volume);
+    free(h->out_deemph);
+    free(h->out_lambda_set);
+    free(h->out_tab);
     delete h;
     return FMB_OK;
 }
@@ -762,6 +892,54 @@ int fmb_set_volume(fmb_handle *h, float volume)
     if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
     h->cfg.volume = volume;
     h->tab.pcm_scale = volume * 32768.0f; /* :717, in float like the reference */
+    for (int s = 0; s < h->cfg.n_streams; ++s) {
+        h->out_volume[s] = volume;
+        h->out_tab[s] = stream_out_entry(h, s);
+    }
+    stream_out_changed(h);
+    return FMB_OK;
+}
+
+int fmb_check_stream_output(int count, const float *volume, const double *deemph, const float *deemph_lambda)
+{
+    for (int i = 0; i < count; ++i) {
+        if (volume && !std::isfinite(volume[i])) return set_err(FMB_ERR_ARG, "volume must be finite");
+        if (deemph && !(std::isfinite(deemph[i]) && deemph[i] >= 0.0))
+            return set_err(FMB_ERR_ARG, "deemph must be a finite time constant >= 0 (0 = off)");
+        if (deemph_lambda && !(deemph_lambda[i] >= 0.0f && deemph_lambda[i] < 1.0f))
+            return set_err(FMB_ERR_ARG, "deemph_lambda must be in [0, 1)");
+    }
+    return FMB_OK;
+}
+
+int fmb_set_stream_output(fmb_handle *h, int first, int count, const float *volume, const double *deemph,
+                          const float *deemph_lambda)
+{
+    if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
+    if (first < 0 || count < 0 || first > h->cfg.n_streams - count) return set_err(FMB_ERR_ARG, "bad stream range");
+    const int rc = fmb_check_stream_output(count, volume, deemph, deemph_lambda);
+    if (rc != FMB_OK) return rc;
+    for (int i = 0; i < count; ++i) {
+        const int s = first + i;
+        if (volume) h->out_volume[s] = volume[i];
+        if (deemph) h->out_deemph[s] = deemph[i];
+        if (deemph_lambda) h->out_lambda_set[s] = deemph_lambda[i];
+        h->out_tab[s] = stream_out_entry(h, s);
+    }
+    stream_out_changed(h);
+    return FMB_OK;
+}
+
+int fmb_get_stream_output(const fmb_handle *h, int first, int count, float *volume, float *lambda, int *deemph_on)
+{
+    if (!h) return set_err(FMB_ERR_ARG, "NULL handle");
+    if (first < 0 || count < 0 || first > h->cfg.n_streams - count) return set_err(FMB_ERR_ARG, "bad stream range");
+    for (int i = 0; i < count; ++i) {
+        const int s = first + i;
+        if (volume) volume[i] = h->out_volume[s];
+        if (lambda) lambda[i] = h->out_tab[s].lambda;
+        if (deemph_on) deemph_on[i] = h->out_tab[s].do_deemph;
+    }
     return FMB_OK;
 }
 
@@ -850,6 +1028,15 @@ const char *fmb_demod_kernel_name(const fmb_handle *h)
                       h->fast / c.rate_out2 == 4 && h->phase / c.rate_out2 == 0;
     if (!ws_kernel_applies(h, dec4)) return "fmb_demod_kernel";
     return "fmb_mono_ws_kernel";
+}
+
+const char *fmb_deemph_kernel_name(const fmb_handle *h)
+{
+    if (!h) return "";
+    int segs = 1, seg_chunks = 0;
+    deemph_segments(h, h->blocks, out_count_for(h, h->phase, h->blocks), &segs, &seg_chunks);
+    if (segs > 1) return h->out_differ ? "fmb_deemph_seg_kernel_per_stream" : "fmb_deemph_seg_kernel";
+    return h->out_differ ? "fmb_deemph_kernel_per_stream" : "fmb_deemph_kernel";
 }
 
 int fmb_sync(fmb_handle *h)

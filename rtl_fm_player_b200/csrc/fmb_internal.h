@@ -33,6 +33,11 @@ typedef struct fmb_tables {
 
 /* Host-side design with glibc sinf/cosf/exp, the reference's float expressions. */
 int fmb_design_tables(const fmb_config *cfg, fmb_tables *t);
+/* The de-emphasis pole of a stream with time constant `deemph` (0 = off: returns 0) and override `deemph_lambda`
+ * (> 0: returned as is) at cfg's output rate; fmb_design_tables takes fmb_tables.lambda from here. */
+float fmb_deemph_pole(const fmb_config *cfg, double deemph, float deemph_lambda);
+/* FMB_OK when count per-stream settings are acceptable to fmb_set_stream_output (NULL array = not given). */
+int fmb_check_stream_output(int count, const float *volume, const double *deemph, const float *deemph_lambda);
 
 /* Kernel geometry (see DESIGN.md "Kernel 1"). */
 #ifndef FMB_NT
@@ -88,6 +93,14 @@ typedef struct fmb_kparams {
 #define FMB_TICKET_SLOTS 4
 #define FMB_LR_BUFS 3              /* decoder-output buffers in rotation (see fmb_handle.d_lr)                  */
 
+/* One stream's output settings as the de-emphasis passes read them: 16 bytes, one vector load per warp. */
+typedef struct fmb_stream_out {
+    float lambda;                  /* de-emphasis pole (unused when do_deemph is 0)       */
+    float pcm_scale;               /* volume * 32768, in float (:717)                     */
+    int do_deemph;
+    int pad;
+} fmb_stream_out;
+
 typedef struct fmb_dparams {
     const float *lr;
     long long lr_pitch;
@@ -108,6 +121,8 @@ typedef struct fmb_dparams {
     float *seg_state;              /* [stream][segs][4]: assumed start (l, r) and end (l, r) of each segment      */
     unsigned int *seg_count;       /* [stream]: segments finished in this pass; the last one walks the junctions
                                       and sets it back to 0                                                       */
+    const fmb_stream_out *out;     /* [stream] per-stream output settings (fmb_set_stream_output), read instead of
+                                      do_deemph / lambda / pcm_scale; NULL: those hold for every stream          */
 } fmb_dparams;
 
 /* Sets fmb_last_error() of the calling thread (host code outside fmb_api.cu reports through it). */

@@ -224,6 +224,57 @@ int fmb_multi_reset(fmb_multi *m)
     return run_all(m, CMD_RESET);
 }
 
+/* streams [first, first+count) of the whole batch: the part on shard g, as its local range and the offset into the
+ * caller's arrays; 0 when the range misses the shard */
+static int shard_part(const fmb_multi *m, int g, int first, int count, int *local_first, int *local_count, int *offset)
+{
+    int sf = 0, sc = 0, lo, hi;
+    fmb_multi_shard_range(m, g, &sf, &sc, NULL);
+    lo = first > sf ? first : sf;
+    hi = first + count < sf + sc ? first + count : sf + sc;
+    if (hi <= lo) return 0;
+    *local_first = lo - sf; *local_count = hi - lo; *offset = lo - first;
+    return 1;
+}
+
+static int bad_range(const fmb_multi *m, int first, int count)
+{
+    return first < 0 || count < 0 || first > m->cfg.n_streams - count;
+}
+
+int fmb_multi_set_stream_output(fmb_multi *m, int first, int count, const float *volume, const double *deemph,
+                                const float *deemph_lambda)
+{
+    int g, rc;
+    if (!m) return fail_arg("NULL handle");
+    if (bad_range(m, first, count)) return fail_arg("bad stream range");
+    /* host bookkeeping only; checked as a whole first, so that no shard is changed when another would refuse */
+    if ((rc = fmb_check_stream_output(count, volume, deemph, deemph_lambda)) != FMB_OK) return rc;
+    for (g = 0; g < m->n; ++g) {
+        int lf, lc, off;
+        if (!shard_part(m, g, first, count, &lf, &lc, &off)) continue;
+        rc = fmb_set_stream_output(m->sh[g].h, lf, lc, volume ? volume + off : NULL, deemph ? deemph + off : NULL,
+                                   deemph_lambda ? deemph_lambda + off : NULL);
+        if (rc != FMB_OK) return rc;
+    }
+    return FMB_OK;
+}
+
+int fmb_multi_get_stream_output(const fmb_multi *m, int first, int count, float *volume, float *lambda, int *deemph_on)
+{
+    int g, rc;
+    if (!m) return fail_arg("NULL handle");
+    if (bad_range(m, first, count)) return fail_arg("bad stream range");
+    for (g = 0; g < m->n; ++g) {
+        int lf, lc, off;
+        if (!shard_part(m, g, first, count, &lf, &lc, &off)) continue;
+        rc = fmb_get_stream_output(m->sh[g].h, lf, lc, volume ? volume + off : NULL, lambda ? lambda + off : NULL,
+                                   deemph_on ? deemph_on + off : NULL);
+        if (rc != FMB_OK) return rc;
+    }
+    return FMB_OK;
+}
+
 int fmb_multi_submit(fmb_multi *m, const uint8_t *iq_host, size_t iq_pitch, int16_t *pcm_host, size_t pcm_pitch, int *ticket)
 {
     int rc;

@@ -100,6 +100,25 @@ class FmMulti:
     def reset(self) -> None:
         L.check(self._lib.fmb_multi_reset(self._m), "fmb_multi_reset")
 
+    def set_stream_output(self, volume=None, deemph=None, deemph_lambda=None, first: int = 0) -> None:
+        """FmBatch.set_stream_output over global stream indices (fmb_multi_set_stream_output)."""
+        count, args = L.stream_output_args(self.cfg.n_streams, first, volume, deemph, deemph_lambda)
+        L.check(self._lib.fmb_multi_set_stream_output(self._m, first, count, *(p for _, p in args)),
+                "fmb_multi_set_stream_output")
+
+    def stream_output(self, first: int = 0, count: int | None = None) -> dict:
+        """FmBatch.stream_output over global stream indices (fmb_multi_get_stream_output)."""
+        count = self.cfg.n_streams - first if count is None else count
+        vol, lam, on = (np.empty(count, np.float32), np.empty(count, np.float32), np.empty(count, np.int32))
+        L.check(self._lib.fmb_multi_get_stream_output(self._m, first, count, vol.ctypes.data_as(C.POINTER(C.c_float)),
+                                                      lam.ctypes.data_as(C.POINTER(C.c_float)),
+                                                      on.ctypes.data_as(C.POINTER(C.c_int))), "fmb_multi_get_stream_output")
+        return {"volume": vol, "lambda": lam, "deemph_on": on.astype(bool)}
+
+    def deemph_kernel_name(self, shard: int = 0) -> str:
+        """The de-emphasis kernel shard `shard`'s next call launches (fmb_deemph_kernel_name)."""
+        return self._lib.fmb_deemph_kernel_name(self.shard_handle(shard)).decode()
+
     def shard_handle(self, g: int) -> int:
         return self._lib.fmb_multi_handle(self._m, g)
 
